@@ -5,6 +5,7 @@ batch 256 per GPU, data-parallel over N B200s).
     python bench.py --gpus N --steps K --warmup W              # our sm_100a path
     python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU path (oracle port)
     python bench.py --workload iw ...                          # IW-1000 evals/s on the 12-layer MNIST model
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs as DIR/*.npy
 
 For N > 1 launch with torch.distributed.run (one rank per GPU).  Rank 0 prints ONE JSON line, last.
 A "step" is one ELBO training step (zero grads, forward, loss, backward, gradient all-reduce,
@@ -336,9 +337,37 @@ def kernel_shares(torch, engine):
         return {"error": repr(e)[:200]}
 
 
+DUMP_SAMPLE = 1 << 20      # entries kept of each dumped array larger than this (a fixed, seeded choice)
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy (float64).  An array of more than DUMP_SAMPLE entries is replaced by the same
+    seeded sample of its flattened entries in every run, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > DUMP_SAMPLE:
+            a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def train_step_outputs(model, out):
+    """What a caller of TrainEngine.step holds after a step: the returned scalars, and the model's updated parameters,
+    their gradients and the BatchNorm running statistics (in the model's own parameter / buffer order)."""
+    import torch
+    params = [p for p in model.parameters() if p.requires_grad]
+    res = {k: v.detach().double().cpu().numpy() for k, v in out.items()}
+    res["params"] = torch.cat([p.detach().flatten() for p in params]).cpu().numpy()
+    res["grads"] = torch.cat([p.grad.detach().flatten() for p in params]).cpu().numpy()
+    res["buffers"] = torch.cat([b.detach().double().flatten() for b in model.buffers()]).cpu().numpy()
+    return res
+
+
 def time_train(cx, cfg_name, batch, dtype, steps, warmup, graph=True, side_streams=3, with_e2e=True, sampler=None,
-               shares=False, dp_check=False):
-    """Build the model, warm up, time `steps` steps device-resident (`value`) and through TrainEngine.step(x_host) (`e2e`)."""
+               shares=False, dp_check=False, dump=None):
+    """Build the model, warm up, time `steps` steps device-resident (`value`) and through TrainEngine.step(x_host) (`e2e`).
+    `dump`: directory that receives what the last device-resident timed step computed (rank 0)."""
     torch = cx.torch
     import lvae_b200
     from lvae_b200.engine import TrainEngine
@@ -367,6 +396,8 @@ def time_train(cx, cfg_name, batch, dtype, steps, warmup, graph=True, side_strea
     cx.barrier()
     clocks = sampler.stop() if sampler is not None else None
     ms = cx.max_over_ranks(e0.elapsed_time(e1)) / steps
+    if dump and cx.rank == 0:
+        dump_outputs(dump, train_step_outputs(model, out))
     res = {"value": batch * cx.world / (ms * 1e-3), "unit": "images/s", "ms_per_step": ms, "steps": steps, "warmup": warmup,
            "dtype": dtype, "per_gpu_batch": batch, "launches_per_step": engine.launches_per_step, "peak_mem_gb": mem_gb,
            "loss": float(out["loss"]), "clocks": clocks}
@@ -455,7 +486,7 @@ def run_dp_check(cx, engine):
             "buckets_flushed_early": [k for k, c in enumerate(engine._ready_counts or []) if c > 0]}
 
 
-def time_iw(cx, batch, K, dtype, steps, warmup, graph=True, full_forward=False, sampler=None):
+def time_iw(cx, batch, K, dtype, steps, warmup, graph=True, full_forward=False, sampler=None, dump=None):
     torch = cx.torch
     import lvae_b200
     from lvae_b200.engine import IWEvaluator, shard_samples
@@ -483,6 +514,8 @@ def time_iw(cx, batch, K, dtype, steps, warmup, graph=True, full_forward=False, 
     cx.barrier()
     clocks = sampler.stop() if sampler is not None else None
     ms = cx.max_over_ranks(e0.elapsed_time(e1)) / steps
+    if dump and cx.rank == 0:
+        dump_outputs(dump, {"iw_bound": res.double().cpu().numpy()})
     value = batch / (ms * 1e-3)                                  # images whose K-sample bound completes per second
     cx.barrier()
     t0 = time.perf_counter()
@@ -532,7 +565,16 @@ def main():
     ap.add_argument("--no-hbm-rooflines", action="store_true", help="skip the stochastic / likelihood kernel microbenchmarks")
     ap.add_argument("--no-extras", action="store_true",
                     help="train workload: skip the iw / configs / value_f32 / dp_check sub-records (A/B timing runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy into a new or empty DIR (float64; arrays of more than %d "
+                         "entries as a fixed seeded sample); the inputs depend on the arguments only" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.dump_outputs and os.path.isdir(args.dump_outputs) and os.listdir(args.dump_outputs):
+        ap.error("--dump-outputs %s is not empty: files of an earlier dump would sit next to this one's" % args.dump_outputs)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -560,7 +602,8 @@ def main():
     side = 0 if args.no_side_stream else args.side_streams
 
     if args.workload == "iw":
-        line = time_iw(cx, batch, args.iw_samples, args.dtype, args.steps, args.warmup, graph, args.iw_full_forward, sampler)
+        line = time_iw(cx, batch, args.iw_samples, args.dtype, args.steps, args.warmup, graph, args.iw_full_forward, sampler,
+                       args.dump_outputs)
         line.update({"vs_baseline": None, "data": "synthetic"})
         if rank == 0 and world == 1 and not args.no_hbm_rooflines:
             line["roofline_hbm"] = hbm_rooflines("iw")
@@ -570,7 +613,7 @@ def main():
         return
 
     main_res = time_train(cx, cfg_name, batch, args.dtype, args.steps, args.warmup, graph, side, True, sampler,
-                          shares=not args.no_extras, dp_check=not args.no_extras)
+                          shares=not args.no_extras, dp_check=not args.no_extras, dump=args.dump_outputs)
     value = main_res["value"]
     gflop = CONV_GFLOP[cfg_name][1]
     line = {"metric": "train images/s (%s LVAE)" % METRIC_NAME.get(cfg_name, cfg_name),

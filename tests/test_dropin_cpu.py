@@ -4,19 +4,23 @@
 dependency.  `LVAEExperiment._make_model` (experiment_manager.py:38-74) then builds OUR LadderVAE from the reference's own
 argparse defaults; its state_dict must have the keys and shapes of the model the reference builds from the same args.
 
-CPU-only (constructing the modules needs no GPU; running them does) and only where the reference tree exists."""
+CPU-only (constructing the modules needs no GPU; running them does).  Importing the reference's experiment layer needs
+the reference tree; the model layout and forward_pass are checked everywhere against tests/golden/reference_checks.npz
+(oracle/make_golden_refchecks.py)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
 from oracle import ref_loader
+from oracle.make_golden_refchecks import DROPIN_KWARGS, FORWARD_PASS_ANNEALS, OUT as REFCHECKS, forward_pass_model
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
+needs_reference = pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
 
 SCRIPT = r'''
 import json, sys, types, argparse
@@ -75,6 +79,7 @@ def run_dropin():
     return json.loads(line[len("RESULT"):])
 
 
+@needs_reference
 def test_reference_experiment_layer_builds_the_kernel_backed_model():
     out = run_dropin()
     ref = ref_loader.REFERENCE_ROOT
@@ -98,9 +103,35 @@ def test_reference_experiment_layer_builds_the_kernel_backed_model():
     assert out["n_opt_params"] == len(list(refm.parameters()))
 
 
+def test_kernel_backed_model_has_the_reference_state_dict_layout():
+    """The LadderVAE the drop-in route builds from ARGV has the state-dict keys, order and shapes, and the parameter
+    count, stored for the reference model built from the same arguments (tests/golden/reference_checks.npz; see
+    oracle/make_golden_refchecks.py for where the stored values come from)."""
+    import lvae_b200
+    g = np.load(REFCHECKS)
+    m = lvae_b200.LadderVAE(**DROPIN_KWARGS)
+    assert [[k, list(v.shape)] for k, v in m.state_dict().items()] == json.loads(str(g["dropin_state_layout"]))
+    assert len(list(m.parameters())) == int(g["dropin_n_params"])
+
+
 def test_restated_forward_pass_matches_the_reference():
-    """tests/dropin_experiment.py restates LVAEExperiment.forward_pass (experiment_manager.py:322-367) for the GPU box,
-    where /root/reference does not exist; here, where it does, both are fed the same model output."""
+    """tests/dropin_experiment.py restates LVAEExperiment.forward_pass (experiment_manager.py:322-367) for machines without
+    the reference tree: against the outputs stored in tests/golden/reference_checks.npz, and, where the reference is
+    present, against the live forward_pass fed the same model output."""
+    from dropin_experiment import forward_pass as restated
+    g = np.load(REFCHECKS)
+    for anneal in FORWARD_PASS_ANNEALS:
+        b = restated(forward_pass_model(), torch.zeros(5, 1, 2, 2), torch.device("cpu"), anneal)
+        assert sorted(b) == list(g["fp%d_keys" % anneal])
+        for k, v in b.items():
+            assert (v is None) == ("fp%d_%s" % (anneal, k) not in g.files), k
+            if v is not None:
+                np.testing.assert_array_equal(v.detach().numpy(), g["fp%d_%s" % (anneal, k)], err_msg=k)
+    if ref_loader.reference_available():
+        _restated_forward_pass_matches_the_live_reference()
+
+
+def _restated_forward_pass_matches_the_live_reference():
     import importlib
     import types
     saved = {k: sys.modules.get(k) for k in ("boilr", "boilr.data", "boilr.nn", "boilr.nn.init", "boilr.utils", "boilr.models",
