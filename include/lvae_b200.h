@@ -132,8 +132,8 @@ typedef struct {
 int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, const float* bias, const float* out_scale,
                       const void* res, void* y, void* y2, int nsplit, int B, int H, int W, int Cin, int N, int ksize,
                       int flip, int out_f32, const LvaeConvFuse* fuse, lvae_stream_t stream);
-/* The tail of a gated residual block as one launch (the default for gated blocks on the bf16 path; LVAE_CONV_GATE_CHAIN=0
- * falls back to conv2 + gate conv as two launches):
+/* The tail of a gated residual block as one launch (gated blocks on the bf16 path whose shapes it serves; the others run
+ * conv2 and the gate conv as two launches):
  *   c2 = (conv3x3(a2) + bias2) * scale2      second 3x3 convolution of lib/nn.py:83-87 with its Dropout2d mask (B,64) or NULL
  *   h  = conv1x1(c2) + bias_g  (128 ch)      GateLayer2d's convolution, lib/nn.py:118
  *   out = act(h[:, :64]) * sigmoid(h[:, 64:]) + x_res          lib/nn.py:121-126 and the residual add :99

@@ -13,16 +13,14 @@
 // (which keeps serving every other convolution).
 #include "common.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
 
-// warp 0 TMA, warp 1 MMA, warps 2 .. 2 + EW - 1 epilogue.  EW = 16 (default): four warps per TMEM lane quadrant, 16 accumulator
-// columns per thread.  The epilogue of this kernel is a serial chain per tile (c2 -> gate GEMM -> gate -> store) that the clock64
-// trace (profiles/trace_conv_gate.py) shows to be latency-bound, not issue-bound: with 8 warps (two per scheduler) a tile took
-// ~4900 cycles at B = 1000 against ~2300 for its MMAs.
-constexpr int CG_EW_DEFAULT = 16;
+// warp 0 TMA, warp 1 MMA, warps 2 .. 2 + EW - 1 epilogue.  The ELU gate runs with EW = 16: four warps per TMEM lane quadrant,
+// 16 accumulator columns per thread (any other activation: EW = 8).  The epilogue of this kernel is a serial chain per tile
+// (c2 -> gate GEMM -> gate -> store) that the clock64 trace (profiles/trace_conv_gate.py) shows to be latency-bound, not
+// issue-bound: with 8 warps (two per scheduler) a tile took ~4900 cycles at B = 1000 against ~2300 for its MMAs.
 constexpr int CG_BM = 128;
 constexpr int CG_TILE_BYTES = CG_BM * 64 * 2;      // 16 KB: one 128-pixel x 64-channel bf16 tile
 constexpr int CG_HALO_BYTES = 18 * 16 * 128;       // 36 KB
@@ -698,9 +696,7 @@ LVAE_API int lvae_conv_gate_tc(const void* a2, const void* w2p, const float* bia
   p.gate_act = gate_act;
   p.store_c2h = c2 ? 1 : 0;
   p.dbg = g_cg_dbg;
-  static int halo_env = -1;
-  if (halo_env < 0) { const char* e = getenv("LVAE_CONV_HALO"); halo_env = e ? atoi(e) : 1; }
-  p.halo = (halo_env && W % 8 == 0 && H % 16 == 0) ? 1 : 0;
+  p.halo = (W % 8 == 0 && H % 16 == 0) ? 1 : 0;
   p.stage_bytes = p.halo ? CG_HALO_BYTES : CG_TILE_BYTES;
   p.tiles_x = W / 8;
   p.tiles_per_img = (W / 8) * (H / 16);
@@ -754,17 +750,13 @@ LVAE_API int lvae_conv_gate_tc(const void* a2, const void* w2p, const float* bia
   static bool attr = false;
   if (!attr) {
     cudaError_t e = cudaFuncSetAttribute(conv_gate_tc_kernel<ACT_ELU, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_gate_tc_kernel<ACT_ELU, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_gate_tc_kernel<-1, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));
     if (e != cudaSuccess) { lvae_set_error("conv_gate_tc: cannot raise dynamic smem: %s", cudaGetErrorString(e)); return LVAE_ERR_CUDA; }
     attr = true;
   }
   const int n_tiles = p.halo ? B * p.tiles_per_img : (p.M_total + CG_BM - 1) / CG_BM;
   const int grid = n_tiles < lvae_num_sms() ? n_tiles : lvae_num_sms();
-  static int ew_env = -1;
-  if (ew_env < 0) { const char* e = getenv("LVAE_CONV_GATE_EW"); ew_env = e ? atoi(e) : CG_EW_DEFAULT; }     // A/B aid: 8 or 16 epilogue warps
-  if (gate_act == ACT_ELU && ew_env == 16) lvae_launch(conv_gate_tc_kernel<ACT_ELU, 16>, grid, 64 + 32 * 16, smem, stream, tmA, tmW2, tmWg, tmC2, tmH, tmOut, p);
-  else if (gate_act == ACT_ELU) lvae_launch(conv_gate_tc_kernel<ACT_ELU, 8>, grid, 64 + 32 * 8, smem, stream, tmA, tmW2, tmWg, tmC2, tmH, tmOut, p);
+  if (gate_act == ACT_ELU) lvae_launch(conv_gate_tc_kernel<ACT_ELU, 16>, grid, 64 + 32 * 16, smem, stream, tmA, tmW2, tmWg, tmC2, tmH, tmOut, p);
   else lvae_launch(conv_gate_tc_kernel<-1, 8>, grid, 64 + 32 * 8, smem, stream, tmA, tmW2, tmWg, tmC2, tmH, tmOut, p);
   LVAE_COUNT_LAUNCH();
   LVAE_CHECK_LAUNCH("conv_gate_tc");

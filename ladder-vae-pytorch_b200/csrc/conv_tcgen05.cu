@@ -19,7 +19,6 @@
 // buffered in TMEM so the epilogue of tile i overlaps the MMAs of tile i+1.
 #include "common.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 #include <mutex>
 
@@ -45,7 +44,7 @@ struct TcParams {
   int tmem_cols;
   // halo mode (3x3, W % 8 == 0, H % 16 == 0): ONE TMA box of 18 rows x 16 columns per 16x8-pixel tile; the nine
   // tap operands are the same shared-memory tile read through shifted UMMA descriptors (no per-tap re-fetch)
-  int halo, stage_bytes, tiles_x, tiles_per_img, bo_mode;
+  int halo, stage_bytes, tiles_x, tiles_per_img;
   // H, W (hence tiles_x, tiles_per_img) are powers of two: the epilogue's per-tile index arithmetic is shifts and masks (the
   // 64-bit m / hw and the tile divisions cost several hundred cycles per tile on the exposed tail of every launch)
   int lg_w, lg_hw, lg_tx, lg_tpi;
@@ -132,15 +131,14 @@ __device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t saddr) {
   d |= (uint64_t)2 << 61;                            // SWIZZLE_128B
   return d;
 }
-// same, with the 8-row groups sbo bytes apart and a start address that is only 128-byte aligned: the swizzle phase
-// of the first row goes into the base-offset field
-__device__ __forceinline__ uint64_t umma_desc_k_sw128_shifted(uint32_t saddr, uint32_t sbo_bytes, int bo_mode) {
+// same, with the 8-row groups sbo bytes apart and a start address that is only 128-byte aligned.  The base-offset field
+// stays zero: the hardware swizzle is a function of the absolute shared-memory address
+__device__ __forceinline__ uint64_t umma_desc_k_sw128_shifted(uint32_t saddr, uint32_t sbo_bytes) {
   uint64_t d = 0;
   d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
   d |= (uint64_t)1 << 16;
   d |= (uint64_t)(sbo_bytes >> 4) << 32;
   d |= (uint64_t)1 << 46;
-  if (bo_mode) d |= (uint64_t)((saddr >> 7) & 7) << 49;
   d |= (uint64_t)2 << 61;
   return d;
 }
@@ -417,7 +415,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             for (int kb = 0; kb < p.n_kb; ++kb) {
               // tap (dy,dx): the tile's first pixel sits at halo row 1+dy, halo column 1+dx; rows are 16 pixels (2048 B)
               const uint32_t a_start = a_base + (uint32_t)(((1 + p.dy[kb]) * 16 + (1 + p.dx[kb])) * 128);
-              const uint64_t adesc = umma_desc_k_sw128_shifted(a_start, 2048, p.bo_mode);
+              const uint64_t adesc = umma_desc_k_sw128_shifted(a_start, 2048);
               const uint64_t bdesc = umma_desc_k_sw128(smem_u32(sW + kb * wbytes_kb));
 #pragma unroll
               for (int k = 0; k < TC_BK / 16; ++k) {
@@ -896,30 +894,20 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   while (p.tmem_cols < 2 * p.Npad) p.tmem_cols *= 2;
   LVAE_REQUIRE(p.tmem_cols <= 512, "conv2d_tc: accumulator does not fit TMEM");
   const int max_smem = 227 * 1024 - 1024 /*align*/ - 8192 /*barriers, bias, BatchNorm table, reduction scratch*/;
-  static int halo_env = -1, bo_env = 0;
-  if (halo_env < 0) {
-    const char* e = getenv("LVAE_CONV_HALO");
-    halo_env = e ? atoi(e) : 1;
-    const char* b = getenv("LVAE_HALO_BO");
-    bo_env = b ? atoi(b) : 0;   // the hardware swizzle is a function of the absolute shared-memory address: no base offset
-  }
   const int wbytes = ((p.n_kb * p.Npad * 128) + 1023) & ~1023;
-  static int tst_env = -1;
-  if (tst_env < 0) { const char* e = getenv("LVAE_CONV_TMA_STORE"); tst_env = e ? atoi(e) : 1; }
-  p.tma_store = (tst_env && !out_f32 && N % 64 == 0 && N <= 128 && !res && (!y2 || nsplit % 64 == 0)) ? 1 : 0;
+  p.tma_store = (!out_f32 && N % 64 == 0 && N <= 128 && !res && (!y2 || nsplit % 64 == 0)) ? 1 : 0;
   const int out_stage = p.tma_store ? (p.Npad / 64 + (p.gate_x ? 1 : 0)) * TC_STAGE_BYTES : 0;
   LVAE_REQUIRE(!p.gate_x || p.tma_store, "conv2d_tc: the gated-residual epilogue needs the TMA-store path");
   LVAE_REQUIRE(!p.fold_gamma || p.tma_store, "conv2d_tc: the folded BatchNorm epilogue needs the TMA-store path");
   LVAE_REQUIRE(!(p.stats_acc || p.bnb_acc) || (p.tma_store && (N == 64 || p.gate_x) && !y2),
                "conv2d_tc: fused reductions need the TMA-store path (bf16 output, N == 64, no residual, no split)");
-  p.halo = (halo_env && ksize == 3 && !x2 && Cin == 64 && W % 8 == 0 && H % 16 == 0 &&
+  p.halo = (ksize == 3 && !x2 && Cin == 64 && W % 8 == 0 && H % 16 == 0 &&
             (max_smem - wbytes - out_stage) / (18 * 16 * 128) >= 2) ? 1 : 0;
   p.stage_bytes = 18 * 16 * 128;
   p.tiles_x = W / 8;
   p.tiles_per_img = (W / 8) * (H / 16);
   set_shifts(p);
-  p.bo_mode = bo_env;
-  LVAE_REQUIRE(!p.pre_gamma || p.halo, "conv2d_tc: the operand-path BatchNorm needs the halo-tile path (LVAE_CONV_HALO)");
+  LVAE_REQUIRE(!p.pre_gamma || p.halo, "conv2d_tc: the operand-path BatchNorm needs the halo-tile path (no shared memory left for two halo stages)");
   int stages = (max_smem - wbytes - out_stage) / (p.halo ? p.stage_bytes : TC_STAGE_BYTES);
   if (stages > 8) stages = 8;
   LVAE_REQUIRE(stages >= 2, "conv2d_tc: weights leave no room for the activation pipeline");

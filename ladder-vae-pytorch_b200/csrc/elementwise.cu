@@ -4,7 +4,6 @@
 // Replaces the ATen elementwise / cuDNN BatchNorm kernels launched by lib/nn.py:50-99,121-126,
 // boilr Interpolate (models/lvae.py:144) and boilr pad/crop (models/lvae.py:176,185).
 #include "common.cuh"
-#include <stdlib.h>
 
 // V-wide (4 or 8 element) typed vector IO: 16-byte transactions for bf16 when V = 8
 template <typename T, int V> __device__ __forceinline__ void ldv(const T* p, float* f);
@@ -1106,12 +1105,9 @@ __global__ void __launch_bounds__(256, GATE ? 2 : 3) bn_act_bwd2_kernel(const T*
 
 // grid whose total thread count is a multiple of C/4, so that every thread keeps the same channel quad
 // Grid of the BatchNorm apply kernels: every CTA re-derives the per-channel table in double precision (FP64 issue rate is
-// 1/64 of FP32 on this part), so fewer, longer-running CTAs win: cap at LVAE_BN_CTAS_PER_SM (default 4) CTAs per SM.
-static inline int bn_grid_cap() {
-  static int cap = 0;
-  if (!cap) { const char* e = getenv("LVAE_BN_CTAS_PER_SM"); cap = e ? atoi(e) : 4; if (cap < 1) cap = 1; }
-  return cap * lvae_num_sms();
-}
+// 1/64 of FP32 on this part), so fewer, longer-running CTAs win: cap at BN_CTAS_PER_SM CTAs per SM.
+constexpr int BN_CTAS_PER_SM = 4;
+static inline int bn_grid_cap() { return BN_CTAS_PER_SM * lvae_num_sms(); }
 // resident CTAs per SM of a kernel at 256 threads (a grid of 4 CTAs per SM for a kernel that fits 3 runs as 1.33 waves)
 template <typename K> static inline int resident_ctas(K kernel) {
   int occ = 0;

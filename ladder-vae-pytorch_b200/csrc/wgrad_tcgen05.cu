@@ -13,7 +13,6 @@
 // Shifted 4-D TMA boxes implement im2col, out-of-bounds zero fill implements the padding.
 #include "common.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace {
@@ -523,19 +522,16 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
   p.tmem_cols = 32;
   while (p.tmem_cols < p.n_pairs * N) p.tmem_cols *= 2;
   p.M_total = B * H * W; p.H = H; p.W = W;
-  static int halo_env = -1;
-  if (halo_env < 0) { const char* e = getenv("LVAE_WGRAD_HALO"); halo_env = e ? atoi(e) : 1; }
   p.in_stride = in_stride;
-  p.halo = (halo_env && in_stride == 1 && ksize == 3 && !x2 && N == 64 && W % 8 == 0 && H % 16 == 0) ? 1 : 0;
+  p.halo = (in_stride == 1 && ksize == 3 && !x2 && N == 64 && W % 8 == 0 && H % 16 == 0) ? 1 : 0;
   p.tiles_x = W / 8;
   p.tiles_per_img = (W / 8) * (H / 16);
   const int n_tiles = p.halo ? B * p.tiles_per_img : (p.M_total + WG_TILE - 1) / WG_TILE;
   // Few, fat CTAs: every CTA pays one pass of reduce-stores over the whole packed gradient (160 KB for a 3x3 conv), so the
   // SM-time of the launch is minimised by giving each CTA several pixel tiles; the kernel runs on a side stream, its latency
-  // does not matter, and the SMs it leaves alone serve the main stream's convolutions (LVAE_WGRAD_TILES_PER_CTA, default 8).
-  static int tpc_env = 0;
-  if (!tpc_env) { const char* e = getenv("LVAE_WGRAD_TILES_PER_CTA"); tpc_env = e ? atoi(e) : 8; if (tpc_env < 1) tpc_env = 1; }
-  int grid = (n_tiles + tpc_env - 1) / tpc_env;
+  // does not matter, and the SMs it leaves alone serve the main stream's convolutions (8: sweep in profiles/tail_kernels_r02.txt).
+  constexpr int WG_TILES_PER_CTA = 8;
+  int grid = (n_tiles + WG_TILES_PER_CTA - 1) / WG_TILES_PER_CTA;
   if (grid > lvae_num_sms()) grid = lvae_num_sms();
   if (grid < 1) grid = 1;
   p.tiles_per_cta = (n_tiles + grid - 1) / grid;

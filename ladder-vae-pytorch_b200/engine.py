@@ -11,7 +11,6 @@ from __future__ import annotations
 
 import ctypes
 import math
-import os
 from typing import Dict, Optional
 
 import torch
@@ -139,7 +138,7 @@ class PackedGradArena:
                 w = m.weight
                 if not (w.requires_grad and hasattr(w, "_lvae_grad_sink")):
                     continue
-                if sp.s2_shape and ops._s2_wgrad_enabled[0]:
+                if sp.s2_shape:
                     # stride-2 resampling convs (lvae_conv2d_wgrad_tc_s2_acc): same packed layout as a 3x3 64 -> 64 conv.  A
                     # ConvTranspose2d's bias gradient sums the large grid (lvae_colsum), not the packed ones-row.
                     n = int(lib.lvae_wgrad_tc_packed_size(64, 3, 0))
@@ -252,7 +251,7 @@ class TrainEngine:
         self.buckets = bucket_ranges_aligned(sorted(self.arena.offsets.values()), self.arena.numel, bucket_bytes)
         # data parallel: bucket k of the gradient arena is all-reduced on the communication stream as soon as the backward has
         # issued its last gradient (the arena is in gradient-ready order), overlapping NCCL with the rest of the backward
-        self.overlap = bool(overlap_allreduce) and self.world > 1 and os.environ.get("LVAE_OVERLAP_ALLREDUCE", "1") != "0"
+        self.overlap = bool(overlap_allreduce) and self.world > 1
         self.comm_stream = torch.cuda.Stream(device=dev) if self.overlap else None
         starts = [s for s, _ in self.buckets]
         import bisect
@@ -271,11 +270,9 @@ class TrainEngine:
         # Side streams run at the lowest priority and the step is captured on a high-priority stream: when SMs free up the
         # block scheduler serves the dependent main chain (fwd / dgrad / BatchNorm) first, the weight gradients fill the rest.
         lo, hi = torch.cuda.Stream.priority_range() if hasattr(torch.cuda.Stream, "priority_range") else (0, -1)
-        # measured: round 1 (two side streams, 18.8 ms step) 19.25 ms with priorities vs 18.83 without; end of round 2 (three side
-        # streams) 14.41-14.44 ms with vs 14.50 without -> on by default; LVAE_STREAM_PRIORITY=0 is the A/B switch
-        prio = os.environ.get("LVAE_STREAM_PRIORITY", "1") != "0"
-        self.side_stream = [torch.cuda.Stream(device=dev, priority=lo if prio else 0) for _ in range(n_side)] if n_side else None
-        self.main_stream = torch.cuda.Stream(device=dev, priority=hi if prio else 0)
+        # measured on a B200 at the end of round 2 (three side streams): 14.41-14.44 ms per step with priorities vs 14.50 without
+        self.side_stream = [torch.cuda.Stream(device=dev, priority=lo) for _ in range(n_side)] if n_side else None
+        self.main_stream = torch.cuda.Stream(device=dev, priority=hi)
         self.graph_fb: Optional[torch.cuda.CUDAGraph] = None
         self.graph_opt: Optional[torch.cuda.CUDAGraph] = None
         self.out: Dict[str, torch.Tensor] = {}

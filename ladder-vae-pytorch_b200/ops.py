@@ -7,9 +7,7 @@ and nothing falls back to ATen for the hot ops; a missing library raises.
 """
 from __future__ import annotations
 
-import contextlib
 import ctypes
-import os
 import struct
 import threading
 from contextlib import contextmanager
@@ -368,9 +366,6 @@ class WeightPack:
 
 
 _tc_enabled = [True]
-_s2_enabled = [os.environ.get("LVAE_CONV_S2_TC", "1") != "0"]
-_debug_skip_wgrad = [os.environ.get("LVAE_DEBUG_SKIP_WGRAD", "0") == "1"]   # measurement aid: main-chain time without weight gradients
-_s2_wgrad_enabled = [os.environ.get("LVAE_WGRAD_S2_TC", "1") != "0"]     # A/B aid: stride-2 weight gradients on tcgen05
 
 
 def set_tensor_cores(flag: bool) -> None:
@@ -422,7 +417,7 @@ class ConvSpec:
 
     def s2_ok(self, t, small_h: int, small_w: int) -> bool:
         """tcgen05 path for the stride-2 convs: bf16 (B,H,W,64) operand, the smaller grid a power of two, W <= 64."""
-        return (_tc_enabled[0] and _s2_enabled[0] and self.s2_shape and t.dtype == torch.bfloat16 and t.shape[3] == 64
+        return (_tc_enabled[0] and self.s2_shape and t.dtype == torch.bfloat16 and t.shape[3] == 64
                 and _pow2(small_h) and _pow2(small_w) and small_w <= 64)
 
     def out_hw(self, h, w):
@@ -477,6 +472,23 @@ def join_side_stream() -> None:
     _side["keep"] = []
 
 
+@contextmanager
+def _wgrad_stream(sunk: bool, keep):
+    """Issue the enclosed weight-gradient launches on the next side stream, after the current stream's work so far, when
+    side streams are set and the gradients go to engine-owned sinks (else on the current stream).  keep: the operands, held
+    until join_side_stream.  Yields the stream slot for packed_grad_log (-1: the current stream)."""
+    sts = _side["streams"]
+    if not (sts and sunk):
+        yield -1
+        return
+    slot = _side["next"] % len(sts)
+    _side["next"] += 1
+    sts[slot].wait_event(torch.cuda.current_stream().record_event())
+    _side["keep"].append(keep)
+    with torch.cuda.stream(sts[slot]):
+        yield slot
+
+
 _wgrad_ws = {}
 stats = {"tc_fwd": 0, "tc_dgrad": 0, "tc_wgrad": 0, "cc_fwd": 0, "cc_dgrad": 0, "cc_wgrad": 0}   # path counters (tests)
 
@@ -489,11 +501,6 @@ def _wgrad_workspace(device) -> torch.Tensor:
         ws = torch.empty(512 * 128, dtype=torch.float32, device=device)        # one packed gradient (<= 5 pairs x 128 x 64)
         _wgrad_ws[key] = ws
     return ws
-
-
-# largest pixel count (B*H*W) for which the per-channel reductions ride in the conv epilogue instead of a pass of their own
-_FUSE_STATS_MAXPIX = int(os.environ.get("LVAE_FUSE_STATS_MAXPIX", str(1 << 40)))
-_FUSE_BNB_MAXPIX = int(os.environ.get("LVAE_FUSE_BNB_MAXPIX", str(1 << 40)))
 
 
 def _tc_fusable(N, out_f32, res, nsplit=0) -> bool:
@@ -582,7 +589,7 @@ def conv_forward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, resn, sta
     if spec.tc_forward_ok(xn, x2n) and (resn is None or resn.dtype == (torch.float32 if want_f32 else torch.bfloat16)):
         wp = spec.pack_tc_fwd.get(weight, torch.bfloat16)
         stats["tc_fwd"] += 1
-        fused = stats_acc is not None and _tc_fusable(spec.cout, want_f32, resn) and _FUSE_STATS_MAXPIX >= xn.shape[0] * xn.shape[1] * xn.shape[2]
+        fused = stats_acc is not None and _tc_fusable(spec.cout, want_f32, resn)
         y = _conv_tc(xn, x2n, wp, bias, out_scale, resn, spec.cout, spec.k, False, want_f32,
                      stats_acc=stats_acc if fused else None)
         return (y, fused) if stats_acc is not None else y
@@ -616,12 +623,11 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
     if padded and not use_tc:
         xn, C1, padded = xn[..., :spec.cin].contiguous(), spec.cin, False
     # stride-2 convs on the tensor cores: dgrad of Conv2d = "transposed" kind over the dy grid, dgrad of ConvTranspose2d =
-    # "gather" kind onto the (smaller) x grid
+    # "gather" kind onto the (smaller) x grid; their weight gradients read the stride-2-shifted operand through an
+    # element-strided tensor map
     hs2, ws2 = (Hi, Wi) if spec.transposed else (Ho, Wo)
-    use_s2 = need_x and x2n is None and spec.s2_shape and spec.s2_ok(gyn, hs2, ws2) and xn.dtype == torch.bfloat16 and C1 == 64
-    # ... and their weight gradients: the stride-2-shifted operand is read through an element-strided tensor map
-    use_s2w = (need_w and x2n is None and spec.s2_shape and spec.s2_ok(gyn, hs2, ws2) and xn.dtype == torch.bfloat16 and C1 == 64
-               and _s2_wgrad_enabled[0])
+    s2 = x2n is None and spec.s2_ok(gyn, hs2, ws2) and xn.dtype == torch.bfloat16 and C1 == 64
+    use_s2, use_s2w = need_x and s2, need_w and s2
     if (use_tc or use_s2 or use_s2w) and out_scale is not None:
         # TMA-fed operands never pass through registers: apply the Dropout2d mask in a separate pass
         gys = torch.empty_like(gyn)
@@ -638,8 +644,7 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
             wpb = spec.pack_tc_bwd.get(weight, torch.bfloat16)
             stats["tc_dgrad"] += 1
             if x2n is None:
-                fuse_bnb = (bnb is not None and not padded and _tc_fusable(spec.cin, False, None)
-                            and _FUSE_BNB_MAXPIX >= gyn.shape[0] * gyn.shape[1] * gyn.shape[2])
+                fuse_bnb = bnb is not None and not padded and _tc_fusable(spec.cin, False, None)
                 # padded (conv_out of a stochastic block reading the 64-channel bf16 copy of z): the gradient goes to the
                 # fp32, Z-channel z the autograd graph holds -> fp32 epilogue, no padding channels
                 gx = _conv_tc(gyn, None, wpb, None, dx_scale, None, spec.cin, spec.k, True, padded,
@@ -665,57 +670,45 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
         gbbuf, bsunk = (None, True)
         if bias is not None and need_b:
             gbbuf, bsunk = _param_grad_buffer(bias)
-        side, slot = None, -1
-        if _side["streams"] and sunk and bsunk:
-            slot = _side["next"] % len(_side["streams"])
-            side = _side["streams"][slot]
-            _side["next"] += 1
-        if side is not None:
-            side.wait_event(torch.cuda.current_stream().record_event())     # gyn is ready
-            _side["keep"].append((xn, x2n, gyn, out_scale))                  # keep operands alive until the join
-            ctx_mgr = torch.cuda.stream(side)
-            ctx_mgr.__enter__()
-        if _debug_skip_wgrad[0]:
-            pass          # timing experiment only (LVAE_DEBUG_SKIP_WGRAD=1): no weight gradients, results are wrong
-        elif use_tc and out_scale is None and C1 == 64 and C2 in (0, 64) and N in (64, 128) and gyn.dtype == torch.bfloat16 \
-                and spec.k * spec.k * (2 if C2 else 1) <= 9:
-            stats["tc_wgrad"] += 1
-            gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
-            if gp is not None:
-                # engine-owned packed gradient: every CTA reduce-adds into it, the engine unpacks them in batched launches
-                _side["log"].setdefault(slot, []).append(weight._lvae_gp_id)
-                call("lvae_conv2d_wgrad_tc_acc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gp.data_ptr(), B, Hi, Wi, N, spec.k,
-                     0, 0, _stream())
+        with _wgrad_stream(sunk and bsunk, (xn, x2n, gyn, out_scale)) as slot:
+            if use_tc and out_scale is None and C1 == 64 and C2 in (0, 64) and N in (64, 128) and gyn.dtype == torch.bfloat16 \
+                    and spec.k * spec.k * (2 if C2 else 1) <= 9:
+                stats["tc_wgrad"] += 1
+                gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
+                if gp is not None:
+                    # engine-owned packed gradient: every CTA reduce-adds into it, the engine unpacks them in batched launches
+                    _side["log"].setdefault(slot, []).append(weight._lvae_gp_id)
+                    call("lvae_conv2d_wgrad_tc_acc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gp.data_ptr(), B, Hi, Wi, N, spec.k,
+                         0, 0, _stream())
+                else:
+                    call("lvae_conv2d_wgrad_tc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gwbuf.data_ptr(), _p(gbbuf),
+                         _wgrad_workspace(xn.device).data_ptr(), B, Hi, Wi, N, spec.k, spec.cin if padded else 0, 0, 0, 0,
+                         _stream())
+            elif use_s2w:
+                stats["tc_wgrad"] += 1
+                big, small = (gyn, xn) if spec.transposed else (xn, gyn)
+                gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
+                if gp is not None:
+                    _side["log"].setdefault(slot, []).append(weight._lvae_gp_id)
+                    call("lvae_conv2d_wgrad_tc_s2_acc", big.data_ptr(), small.data_ptr(), gp.data_ptr(), B, hs2, ws2, _stream())
+                else:
+                    call("lvae_conv2d_wgrad_tc_s2", big.data_ptr(), small.data_ptr(), gwbuf.data_ptr(),
+                         None if spec.transposed else _p(gbbuf), _wgrad_workspace(xn.device).data_ptr(), B, hs2, ws2, _stream())
+                if spec.transposed and gbbuf is not None:      # the bias gradient sums the large grid
+                    call("lvae_colsum", gyn.data_ptr(), None, gbbuf.data_ptr(), B, Ho * Wo, N, _dt(gyn), _stream())
+            elif not spec.transposed:
+                stats["cc_wgrad"] += 1
+                call("lvae_conv2d_wgrad", xn.data_ptr(), _p(x2n), gyn.data_ptr(), None, _p(out_scale),
+                     gwbuf.data_ptr(), _p(gbbuf), B, Hi, Wi, C1, C2, Ho, Wo, N, spec.k, spec.k, spec.stride,
+                     spec.pad, _dt(xn), _stream())
             else:
-                call("lvae_conv2d_wgrad_tc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gwbuf.data_ptr(), _p(gbbuf),
-                     _wgrad_workspace(xn.device).data_ptr(), B, Hi, Wi, N, spec.k, spec.cin if padded else 0, 0, 0, 0, _stream())
-        elif use_s2w:
-            stats["tc_wgrad"] += 1
-            big, small = (gyn, xn) if spec.transposed else (xn, gyn)
-            gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
-            if gp is not None:
-                _side["log"].setdefault(slot, []).append(weight._lvae_gp_id)
-                call("lvae_conv2d_wgrad_tc_s2_acc", big.data_ptr(), small.data_ptr(), gp.data_ptr(), B, hs2, ws2, _stream())
-            else:
-                call("lvae_conv2d_wgrad_tc_s2", big.data_ptr(), small.data_ptr(), gwbuf.data_ptr(),
-                     None if spec.transposed else _p(gbbuf), _wgrad_workspace(xn.device).data_ptr(), B, hs2, ws2, _stream())
-            if spec.transposed and gbbuf is not None:      # the bias gradient sums the large grid
-                call("lvae_colsum", gyn.data_ptr(), None, gbbuf.data_ptr(), B, Ho * Wo, N, _dt(gyn), _stream())
-        elif not spec.transposed:
-            stats["cc_wgrad"] += 1
-            call("lvae_conv2d_wgrad", xn.data_ptr(), _p(x2n), gyn.data_ptr(), None, _p(out_scale),
-                 gwbuf.data_ptr(), _p(gbbuf), B, Hi, Wi, C1, C2, Ho, Wo, N, spec.k, spec.k, spec.stride,
-                 spec.pad, _dt(xn), _stream())
-        else:
-            # roles swap: "input" = dy (scaled), "output grad" = x; result is (Cin, Cout, k, k)
-            stats["cc_wgrad"] += 1
-            call("lvae_conv2d_wgrad", gyn.data_ptr(), None, xn.data_ptr(), _p(out_scale), None,
-                 gwbuf.data_ptr(), None, B, Ho, Wo, N, 0, Hi, Wi, C1, spec.k, spec.k, spec.stride, spec.pad,
-                 _dt(xn), _stream())
-            if gbbuf is not None:
-                call("lvae_colsum", gyn.data_ptr(), _p(out_scale), gbbuf.data_ptr(), B, Ho * Wo, N, _dt(gyn), _stream())
-        if side is not None:
-            ctx_mgr.__exit__(None, None, None)
+                # roles swap: "input" = dy (scaled), "output grad" = x; result is (Cin, Cout, k, k)
+                stats["cc_wgrad"] += 1
+                call("lvae_conv2d_wgrad", gyn.data_ptr(), None, xn.data_ptr(), _p(out_scale), None,
+                     gwbuf.data_ptr(), None, B, Ho, Wo, N, 0, Hi, Wi, C1, spec.k, spec.k, spec.stride, spec.pad,
+                     _dt(xn), _stream())
+                if gbbuf is not None:
+                    call("lvae_colsum", gyn.data_ptr(), _p(out_scale), gbbuf.data_ptr(), B, Ho * Wo, N, _dt(gyn), _stream())
         gw = None if sunk else gwbuf
         gb = None if (bsunk or gbbuf is None) else gbbuf
     return gx, gx2, gw, gb
@@ -845,13 +838,16 @@ def bn_act(x, bn, act_id: int, out_dtype=None):
 BN_STRIPES = 8
 _bn_epoch = [0]
 _whole_block = [True]
-_gate_fused = [os.environ.get("LVAE_GATE_FUSED", "1") != "0"]
 _gate_keep_h = [True]     # set per call by gated_block(): autograd.Function.forward always runs with grad mode off
-# conv2 + gate conv + gate as ONE launch, the 1x1 GEMM reading the staged conv2 tile (lvae_conv_gate_tc; validated and
-# timed on the B200 in round 2: bit-identical tensors, 17.41 -> 16.71 ms per CIFAR-15 step).  LVAE_CONV_GATE_CHAIN=0 = A/B.
-_gate_chain = [os.environ.get("LVAE_CONV_GATE_CHAIN", "1") != "0"]
-_eval_bn_pre = [os.environ.get("LVAE_EVAL_BN_PRE", "1") != "0"]      # A/B aid: eval-mode BatchNorm1 on conv1's operand path
-_eval_bn_fold = [os.environ.get("LVAE_EVAL_BN_FOLD", "1") != "0"]    # A/B aid: eval-mode BatchNorm2 folded into conv1's epilogue
+# Fused paths of the gated blocks.  Always on: they are flags only so that tests/test_conv_gate_gpu.py and
+# tests/test_block_stack_fusion_gpu.py can turn them off for their reference runs.
+# _gate_chain: conv2 + gate conv + gate as ONE launch, the 1x1 GEMM reading the staged conv2 tile (lvae_conv_gate_tc; on a
+# B200 in round 2: bit-identical tensors, 17.41 -> 16.71 ms per CIFAR-15 step).  _eval_bn_pre / _eval_bn_fold: eval-mode
+# BatchNorm1 on conv1's operand path / BatchNorm2 folded into conv1's epilogue.  _stack_fusion: see below.
+_gate_chain = [True]
+_eval_bn_pre = [True]
+_eval_bn_fold = [True]
+_stack_fusion = [True]
 
 
 def _conv_gate_chain(a2, w2p, bias2, mask2, wgp, gbias, xn, gact, stats_acc, keep):
@@ -888,7 +884,6 @@ def new_forward_epoch() -> int:
 # apply over instead of launching it (keyed by the storage of the dx tensor it returns); block k-1 runs both as one kernel
 # (lvae_bn_act_bwd2_gate).  Only when the stack guarantees that block k is the sole consumer of block k-1's output -- the
 # gradient then reaches block k-1 unaccumulated, as the same tensor -- and only with engine-owned gradient sinks.
-_stack_fusion = [os.environ.get("LVAE_BLOCK_STACK_FUSION", "1") != "0"]
 _private_out = [False]
 _defer_bn1_next = [False]
 _pending_bn1 = {}
@@ -904,7 +899,7 @@ def check_no_pending_bn1() -> None:
         n = len(_pending_bn1)
         _pending_bn1.clear()
         raise RuntimeError("lvae_b200: %d deferred BatchNorm-backward apply pass(es) were never picked up by the preceding "
-                           "block's backward: their input gradients were not computed (set LVAE_BLOCK_STACK_FUSION=0)" % n)
+                           "block's backward: their input gradients were not computed (cross-block fusion, ops._stack_fusion)" % n)
 
 
 def bn_scratch(bn, device):
@@ -1008,7 +1003,7 @@ class GatedBlockFn(Function):
             stats["gate_chain"] = stats.get("gate_chain", 0) + 1
             y2, h, out = _conv_gate_chain(a2, conv2.spec.pack_tc_fwd.get(w2, torch.bfloat16), cb2, m2,
                                           gspec.pack_tc_fwd.get(wg, torch.bfloat16), gbias, xn, gact, out_stats, _gate_keep_h[0])
-        elif (_gate_fused[0] and C == 64 and gspec.cout == 128 and xn.dtype == torch.bfloat16 and not gspec.out_fp32
+        elif (C == 64 and gspec.cout == 128 and xn.dtype == torch.bfloat16 and not gspec.out_fp32
                 and gspec.tc_forward_ok(y2, None)):
             # gate, residual add and the output statistics ride in the epilogue of the 1x1 gate conv
             stats["tc_fwd"] += 1
@@ -1229,13 +1224,10 @@ class CropFn(Function):
         return as_nchw(dx), None
 
 
-_crop_view = [os.environ.get("LVAE_CROP_VIEW", "1") != "0"]      # A/B aid
-
-
 def crop(x, size):
     if tuple(x.shape[2:]) == tuple(int(s) for s in size):
         return x
-    if _crop_view[0] and not torch.is_grad_enabled() and x.is_cuda:
+    if not torch.is_grad_enabled() and x.is_cuda:
         # nothing runs backward (IW evaluator, sampling): the centred crop is a strided view of the NHWC buffer -- the Bernoulli
         # head's narrow conv reads the window in place, any other consumer makes it contiguous itself (ops.nhwc)
         xn = x.permute(0, 2, 3, 1)
@@ -1556,13 +1548,7 @@ class DmolHeadFn(Function):
         if ctx.needs_input_grad[1]:
             gwbuf, sunk = _param_grad_buffer(weight)
             gbbuf, bsunk = _param_grad_buffer(bias)
-            side = None
-            if _side["streams"] and sunk and bsunk:
-                side = _side["streams"][_side["next"] % len(_side["streams"])]
-                _side["next"] += 1
-                side.wait_event(torch.cuda.current_stream().record_event())
-                _side["keep"].append((hn, dl))
-            with (torch.cuda.stream(side) if side is not None else contextlib.nullcontext()):
+            with _wgrad_stream(sunk and bsunk, (hn, dl)):
                 stats["tc_wgrad"] += 1
                 # five accumulator pairs x 128 columns would not fit TMEM: two launches over 64 output channels each
                 taps = spec.k * spec.k
