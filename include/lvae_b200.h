@@ -63,7 +63,9 @@ int lvae_conv2d_tc(const void* x, const void* x2, const void* wp, const float* b
 /* bf16 tensor-core weight gradient for the same convolutions (reduction over pixels, MN-major operands,
  * two filter taps per M = 128 MMA, bias gradient from an all-ones operand block): x, x2 (B,H,W,64) bf16,
  * dy (B,H,W,N) bf16 with N in {64,128} (already multiplied by the Dropout2d mask); dw (N,I,k,k) fp32 +=,
- * dbias [N] += or NULL; ws = lvae_wgrad_tc_workspace(...) floats of scratch (one packed gradient, see below). */
+ * dbias [N] += or NULL; ws = lvae_wgrad_tc_workspace(...) floats of scratch (one packed gradient, see below).
+ * I_real: input channels of dw (0 = 64 per input, at most that); N_real: rows of dw (0 = N, at most N);
+ * dy carries dyC channels (0 = N), of which channels [dy_c0, dy_c0 + N) are used (dy_c0 a multiple of 64). */
 int lvae_conv2d_wgrad_tc(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws, int B,
                          int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0, lvae_stream_t stream);
 long long lvae_wgrad_tc_workspace(int B, int H, int W, int N, int ksize, int two_inputs);

@@ -467,6 +467,12 @@ static bool wgrad_shape_ok(int N, int ksize, int inputs) {
   return n_pairs <= WG_MAX_PAIRS && n_pairs * N <= 512;
 }
 
+// I_real / N_real (0 = all) select the rows / columns of Gp the unpack reads: more than the packed gradient holds would read
+// (and with the clear bit zero) memory past each Gp row, or copy never-written shared memory into dw.
+static bool wgrad_real_ok(int N, int inputs, int I_real, int N_real) {
+  return I_real >= 0 && I_real <= 64 * inputs && N_real >= 0 && N_real <= N;
+}
+
 // Floats in the packed gradient Gp of one convolution (0 if the shape is unsupported): pairs x 128 rows x N columns.
 LVAE_API long long lvae_wgrad_tc_packed_size(int N, int ksize, int two_inputs) {
   const int inputs = two_inputs ? 2 : 1;
@@ -503,7 +509,10 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
                              int ksize, int dyC, int dy_c0, int in_stride, cudaStream_t stream) {
   LVAE_REQUIRE(x && dy && gp, "conv2d_wgrad_tc: null pointer");
   LVAE_REQUIRE((N == 64 || N == 128) && (ksize == 1 || ksize == 3), "conv2d_wgrad_tc: N must be 64 or 128, ksize 1 or 3");
-  LVAE_REQUIRE((W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W <= 128, "conv2d_wgrad_tc: H and W must be powers of two (W <= 128)");
+  LVAE_REQUIRE(B > 0 && H > 0 && W > 0 && (W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W <= 128,
+               "conv2d_wgrad_tc: H and W must be powers of two (W <= 128), B positive");
+  if (dyC <= 0) dyC = N;
+  LVAE_REQUIRE(dy_c0 >= 0 && dy_c0 % 64 == 0 && dy_c0 + N <= dyC, "conv2d_wgrad_tc: bad dY channel window");
   EncodeTiledFn enc = wg_get_encode();
   if (!enc) { lvae_set_error("conv2d_wgrad_tc: cuTensorMapEncodeTiled unavailable"); return LVAE_ERR_CUDA; }
   const int inputs = x2 ? 2 : 1, taps = ksize * ksize;
@@ -545,8 +554,6 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
   int r = p.halo ? make_act_map(enc, &tmX, x, B, H, W, 64, 16, 18, 1)
                  : make_act_map(enc, &tmX, x, B, H * in_stride, W * in_stride, 64, bw, bh, bn, in_stride);
   if (!r) r = make_act_map(enc, &tmX2, x2 ? x2 : x, B, H, W, 64, bw, bh, bn);
-  if (dyC <= 0) dyC = N;
-  LVAE_REQUIRE(dy_c0 % 64 == 0 && dy_c0 + N <= dyC, "conv2d_wgrad_tc: bad dY channel window");
   p.dy_c0 = dy_c0;
   if (!r) r = make_act_map(enc, &tmDY, dy, B, H, W, dyC, bw, bh, bn);
   if (!r) {
@@ -579,6 +586,8 @@ LVAE_API int lvae_wgrad_unpack_desc(void* desc_host, const float* gp, float* dw,
                                     int I_real, int N_real, int clear) {
   LVAE_REQUIRE(desc_host && gp && dw, "wgrad_unpack_desc: null pointer");
   LVAE_REQUIRE(wgrad_shape_ok(N, ksize, two_inputs ? 2 : 1), "wgrad_unpack_desc: unsupported shape");
+  LVAE_REQUIRE(wgrad_real_ok(N, two_inputs ? 2 : 1, I_real, N_real),
+               "wgrad_unpack_desc: I_real %d / N_real %d outside 0..%d / 0..%d", I_real, N_real, two_inputs ? 128 : 64, N);
   fill_unpack_desc((UnpackDesc*)desc_host, gp, dw, dbias, N, ksize, two_inputs ? 2 : 1, I_real, N_real, clear);
   return LVAE_OK;
 }
@@ -617,6 +626,8 @@ LVAE_API int lvae_conv2d_wgrad_tc(const void* x, const void* x2, const void* dy,
   LVAE_REQUIRE(x && dy && dw && ws, "conv2d_wgrad_tc: null pointer");
   const long long n = lvae_wgrad_tc_packed_size(N, ksize, x2 != nullptr);
   LVAE_REQUIRE(n > 0, "conv2d_wgrad_tc: unsupported shape");
+  LVAE_REQUIRE(wgrad_real_ok(N, x2 ? 2 : 1, I_real, N_real),
+               "conv2d_wgrad_tc: I_real %d / N_real %d outside 0..%d / 0..%d", I_real, N_real, x2 ? 128 : 64, N);
   cudaError_t e = cudaMemsetAsync(ws, 0, (size_t)n * 4, stream);
   if (e != cudaSuccess) { lvae_set_error("conv2d_wgrad_tc: memset failed: %s", cudaGetErrorString(e)); return LVAE_ERR_CUDA; }
   int rc = lvae_conv2d_wgrad_tc_acc(x, x2, dy, ws, B, H, W, N, ksize, dyC, dy_c0, stream);

@@ -145,13 +145,16 @@ class PackedGradArena:
                     if m.bias is None or hasattr(m.bias, "_lvae_grad_sink"):
                         convs.append((m, False, n))
                     continue
-                if not (sp.tc_shape and sp.cout in (64, 128)):
+                if not sp.tc_shape:
                     continue
                 two = sp.cin == 128 and sp.k == 1
                 if not (sp.cin <= 64 or two):
                     continue
+                # only convs whose weight gradient is one launch (ops.conv_backward_raw splits the others over dY windows)
+                if ops.wgrad_tc_plan(sp.cout, sp.k, two) != ((sp.cout, 0),):
+                    continue
                 n = int(lib.lvae_wgrad_tc_packed_size(sp.cout, sp.k, int(two)))
-                if n > 0 and (m.bias is None or hasattr(m.bias, "_lvae_grad_sink")):
+                if m.bias is None or hasattr(m.bias, "_lvae_grad_sink"):
                     convs.append((m, two, n))
         self.n = len(convs)
         if not self.n:

@@ -503,6 +503,29 @@ def _wgrad_workspace(device) -> torch.Tensor:
     return ws
 
 
+_wgrad_tc_fits = {}
+
+
+def wgrad_tc_plan(N: int, k: int, two_inputs: bool):
+    """Launches ((width, first dY channel), ...) of the tensor-core weight gradient of a stride-1 conv with N in {64, 128}
+    output channels, or () when the kernel cannot take it.  What fits is the library's own rule
+    (lvae_wgrad_tc_packed_size > 0); a 3x3 conv with N = 128 does not fit TMEM and runs as two launches over 64-channel
+    windows of dY.  PackedGradArena gives a packed gradient exactly to the single-launch shapes."""
+    def fits(n):
+        key = (n, k, bool(two_inputs))
+        ok = _wgrad_tc_fits.get(key)
+        if ok is None:
+            ok = _wgrad_tc_fits[key] = int(_capi.lib().lvae_wgrad_tc_packed_size(n, k, int(bool(two_inputs)))) > 0
+        return ok
+    if N not in (64, 128):
+        return ()
+    if fits(N):
+        return ((N, 0),)
+    if N == 128 and fits(64):
+        return ((64, 0), (64, 64))
+    return ()
+
+
 def _tc_fusable(N, out_f32, res, nsplit=0) -> bool:
     """Can the conv's epilogue carry a fused per-channel reduction (TMA-store path of lvae_conv2d_tc)?"""
     return N == 64 and not out_f32 and res is None and not nsplit
@@ -670,20 +693,25 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
         gbbuf, bsunk = (None, True)
         if bias is not None and need_b:
             gbbuf, bsunk = _param_grad_buffer(bias)
+        plan = wgrad_tc_plan(N, spec.k, C2 > 0) if (use_tc and out_scale is None and C1 == 64 and C2 in (0, 64)
+                                                     and gyn.dtype == torch.bfloat16) else ()
         with _wgrad_stream(sunk and bsunk, (xn, x2n, gyn, out_scale)) as slot:
-            if use_tc and out_scale is None and C1 == 64 and C2 in (0, 64) and N in (64, 128) and gyn.dtype == torch.bfloat16 \
-                    and spec.k * spec.k * (2 if C2 else 1) <= 9:
+            if plan:
                 stats["tc_wgrad"] += 1
                 gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
                 if gp is not None:
                     # engine-owned packed gradient: every CTA reduce-adds into it, the engine unpacks them in batched launches
+                    assert plan == ((N, 0),), "packed gradient of a conv whose weight gradient is split"
                     _side["log"].setdefault(slot, []).append(weight._lvae_gp_id)
                     call("lvae_conv2d_wgrad_tc_acc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gp.data_ptr(), B, Hi, Wi, N, spec.k,
                          0, 0, _stream())
                 else:
-                    call("lvae_conv2d_wgrad_tc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gwbuf.data_ptr(), _p(gbbuf),
-                         _wgrad_workspace(xn.device).data_ptr(), B, Hi, Wi, N, spec.k, spec.cin if padded else 0, 0, 0, 0,
-                         _stream())
+                    # a split launch covers output channels [c0, c0 + n): rows c0.. of dw (N, cin, k, k) and of dbias
+                    row = spec.cin * spec.k * spec.k * 4
+                    for n, c0 in plan:
+                        call("lvae_conv2d_wgrad_tc", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gwbuf.data_ptr() + c0 * row,
+                             None if gbbuf is None else gbbuf.data_ptr() + c0 * 4, _wgrad_workspace(xn.device).data_ptr(),
+                             B, Hi, Wi, n, spec.k, spec.cin if padded else 0, 0, N, c0, _stream())
             elif use_s2w:
                 stats["tc_wgrad"] += 1
                 big, small = (gyn, xn) if spec.transposed else (xn, gyn)
