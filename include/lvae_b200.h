@@ -53,8 +53,8 @@ int lvae_conv2d_gather(const void* x, const void* x2, const void* wp, const floa
 int lvae_conv2d_wgrad(const void* u, const void* u2, const void* dz, const float* in_scale, const float* out_scale,
                       float* dw, float* dbias, int B, int Hi, int Wi, int C1, int C2, int Ho, int Wo, int O, int kh,
                       int kw, int stride, int pad, int dtype, lvae_stream_t stream);
-/* bf16 tensor-core path (TMA -> tcgen05.mma -> TMEM) for the stride-1 "same" convs with 64 channels per
- * input tensor: x, x2 (B,H,W,64) bf16; wp = lvae_pack_weights mode 2 (forward) / 3 (dgrad, flip = 1);
+/* bf16 tensor-core path (TMA -> tcgen05.mma -> TMEM) for the stride-1 "same" convs with a multiple of 64 (at most
+ * 256) channels per input tensor, two inputs of equal width: x, x2 (B,H,W,Cin) bf16; wp = lvae_pack_weights mode 2 (forward) / 3 (dgrad, flip = 1);
  * y (B,H,W,N) bf16 or fp32 (out_f32); y2 != NULL splits the N output columns at nsplit (dgrad of the
  * two-input merge conv).  H, W powers of two, W <= 128, N <= 256, ksize 1 or 3. */
 int lvae_conv2d_tc(const void* x, const void* x2, const void* wp, const float* bias, const float* out_scale,
@@ -69,6 +69,13 @@ int lvae_conv2d_tc(const void* x, const void* x2, const void* wp, const float* b
 int lvae_conv2d_wgrad_tc(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws, int B,
                          int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0, lvae_stream_t stream);
 long long lvae_wgrad_tc_workspace(int B, int H, int W, int N, int ksize, int two_inputs);
+/* The same over a 64-channel window of wider inputs: x, x2 (B,H,W,xC) bf16 (xC a multiple of 64 up to 256; 0 = 64), of
+ * which channels [x_c0, x_c0 + 64) are read (x_c0 a multiple of 64).  dw (N_real, I_real, k, k) with I_real = xC per input
+ * (0) or fewer; this launch adds input channels s * xC + x_c0 + [0, 64) of input s.  Every launch also adds the bias
+ * gradient, so a caller splitting one conv over several X windows passes dbias to one of them per dY window. */
+int lvae_conv2d_wgrad_tc_ex(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws, int B,
+                            int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0, int xC, int x_c0,
+                            lvae_stream_t stream);
 /* The same gradient in two steps, for callers that batch the re-layout (engine.py: one unpack launch per training step
  * instead of one per convolution; replaces the per-parameter `.grad` accumulation of loss.backward(),
  * experiment_manager.py:78-80 / boilr's training loop).  lvae_conv2d_wgrad_tc_acc ADDS the gradient into the packed
@@ -134,6 +141,10 @@ typedef struct {
 int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, const float* bias, const float* out_scale,
                       const void* res, void* y, void* y2, int nsplit, int B, int H, int W, int Cin, int N, int ksize,
                       int flip, int out_f32, const LvaeConvFuse* fuse, lvae_stream_t stream);
+/* How lvae_conv2d_tc[_ex] holds the weights of a shape, decided by the code the launch uses (pure host, no CUDA call):
+ * 0 = rejected, 1 = resident (all k-blocks stay in shared memory; the fused epilogues and halo tiles need this),
+ * 2 = streamed (each pipeline stage carries its k-block's weight tile next to the activation box; plain epilogues). */
+int lvae_conv2d_tc_plan(int Cin, int N, int ksize, int two_inputs, int H, int W, int out_f32);
 /* The tail of a gated residual block as one launch (gated blocks on the bf16 path whose shapes it serves; the others run
  * conv2 and the gate conv as two launches):
  *   c2 = (conv3x3(a2) + bias2) * scale2      second 3x3 convolution of lib/nn.py:83-87 with its Dropout2d mask (B,64) or NULL

@@ -29,6 +29,7 @@ _SIGNATURES = {
     "lvae_conv3x3_narrow_ex": [P, P, P, P, I, I, I, I, I, I, L, P],
     "lvae_channel_scale": [P, P, P, I, I, I, I, P],
     "lvae_conv2d_wgrad_tc": [P, P, P, P, P, P, I, I, I, I, I, I, I, I, I, P],
+    "lvae_conv2d_wgrad_tc_ex": [P, P, P, P, P, P, I, I, I, I, I, I, I, I, I, I, I, P],
     "lvae_conv2d_wgrad_tc_acc": [P, P, P, P, I, I, I, I, I, I, I, P],
     "lvae_conv2d_wgrad_tc_s2_acc": [P, P, P, I, I, I, P],
     "lvae_conv2d_wgrad_tc_s2": [P, P, P, P, P, I, I, I, P],
@@ -82,6 +83,7 @@ _SPECIAL = {
     "lvae_get_pdl": ([], c_int),
     "lvae_wgrad_tc_workspace": ([I, I, I, I, I, I], c_longlong),
     "lvae_wgrad_tc_packed_size": ([I, I, I], c_longlong),
+    "lvae_conv2d_tc_plan": ([I, I, I, I, I, I, I], c_int),
     "lvae_wgrad_unpack_desc_size": ([], c_int),
     "lvae_stoch_ws_bytes": ([I], c_longlong),
 }

@@ -12,7 +12,10 @@
 // pixels is ONE 4-D TMA box {64 ch, bw, bh, bn}; shifting the box origin by the tap offset
 // implements im2col, and TMA's out-of-bounds zero fill implements the zero padding (the batch is
 // its own tensor dimension, so a shifted box never bleeds into the neighbouring image).
-// All taps' weights stay resident in shared memory for the lifetime of a persistent CTA.
+// All taps' weights stay resident in shared memory for the lifetime of a persistent CTA when they leave room for at least
+// two activation stages ("resident").  Wider layers (3x3 128 -> 128 is 288 KB of weights) stream them instead: each
+// pipeline stage then carries the A box of a k-block and the matching [Npad][64] weight tile, landing on one barrier
+// ("streamed", plain epilogues only).  tc_weight_plan decides from the shape alone; lvae_conv2d_tc_plan exposes it.
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + single-thread MMA
 // issuer, warps 2..9 = epilogue (TMEM lane quadrant = warp_id % 4, two warps per quadrant split the columns).  The accumulator is double
@@ -267,7 +270,8 @@ __device__ __forceinline__ void epilogue16(const uint32_t* __restrict__ r, const
 // fp32 epilogue (90 vs 51 us for the 64 -> 100 head).
 // ACT (FUSE 2 / 3 only): the activation of the fused BatchNorm-backward / gate pass as a compile-time constant (ACT_ELU, the
 // model default) or -1 = runtime value; a switch inside the unrolled second pass costs one jump table per element.
-template <int FUSE, int ACT = -1>
+// SW: streamed weights (FUSE == 0, non-halo tiles only): no resident weight block, stage = A box + B tile.
+template <int FUSE, int ACT = -1, bool SW = false>
 __global__ void __launch_bounds__(FUSE == 4 ? TC_THREADS + 160 : TC_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
                const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmY,
@@ -277,9 +281,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
   // (offset arithmetic on the __shared__ array, not on a uintptr_t: the compiler keeps the shared address space)
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int wbytes_kb = p.Npad * 128;                        // one k-block of weights
-  uint8_t* sW = smem;                                        // n_kb * Npad * 128
-  uint8_t* sA = sW + ((p.n_kb * wbytes_kb + 1023) & ~1023);  // n_stages * 16 KB
-  const int stage_bytes = p.halo ? p.stage_bytes : TC_STAGE_BYTES;
+  uint8_t* sW = smem;                                        // n_kb * Npad * 128 (resident weights only)
+  uint8_t* sA = sW + (SW ? 0 : ((p.n_kb * wbytes_kb + 1023) & ~1023));  // n_stages * stage_bytes
+  const int stage_bytes = p.halo ? p.stage_bytes : (SW ? TC_STAGE_BYTES + wbytes_kb : TC_STAGE_BYTES);
   uint8_t* sOut = sA + p.n_stages * stage_bytes;             // (N/64) x 16 KB output staging (TMA-store epilogue only)
   uint64_t* bars = (uint64_t*)(sOut + (p.tma_store ? (p.Npad / 64 + (FUSE == 3 ? 1 : 0)) * TC_STAGE_BYTES : 0));
   // barrier layout: [0..S) full, [S..2S) empty, 2S: weights, 2S+1..2S+2: tmem_full[2], 2S+3..2S+4: tmem_empty[2]
@@ -311,7 +315,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     if (FUSE == 4) for (int i = 0; i < S; ++i) mbar_init(BAR(2 * S + 5 + i), 5);     // one arrive per transform warp
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 0) {
+  if (warp == 0 && !SW) {
     __syncwarp();
     // weights were packed many kernels ago: fetch them before waiting on the previous kernel (PDL prologue)
     if (elect_one()) {
@@ -377,9 +381,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
         for (int kb = 0; kb < p.n_kb; ++kb) {
           mbar_wait(BAR(S + stage), phase ^ 1);
           if (elect_one()) {
-            mbar_expect_tx(BAR(stage), TC_STAGE_BYTES);
-            tma_load_4d(smem_u32(sA + stage * TC_STAGE_BYTES), p.src[kb] ? &tmA1 : &tmA0, BAR(stage), 64 * p.coff[kb],
+            uint8_t* dst = sA + stage * (SW ? stage_bytes : TC_STAGE_BYTES);
+            mbar_expect_tx(BAR(stage), SW ? (uint32_t)stage_bytes : (uint32_t)TC_STAGE_BYTES);
+            tma_load_4d(smem_u32(dst), p.src[kb] ? &tmA1 : &tmA0, BAR(stage), 64 * p.coff[kb],
                         w0 + p.dx[kb], h0 + p.dy[kb], n0);
+            // streamed weights: this k-block's [Npad][64] tile lands behind the A box, on the same barrier
+            if (SW) tma_load_2d(smem_u32(dst + TC_STAGE_BYTES), &tmW, BAR(stage), 0, (p.use_wblk ? p.wblk[kb] : kb) * p.Npad);
           }
           __syncwarp();
           if (++stage == S) { stage = 0; phase ^= 1; }
@@ -394,7 +401,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
       // instruction descriptor: D fp32, A/B bf16, both K-major, M = 128, N = Npad
       const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.Npad >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      mbar_wait(BAR(2 * S), 0);
+      if (!SW) mbar_wait(BAR(2 * S), 0);
       tc_fence_after();
       int stage = 0;
       uint32_t phase = 0;
@@ -434,8 +441,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
           mbar_wait(BAR(stage), phase);
           tc_fence_after();
           if (elect_one()) {
-            const uint64_t adesc = umma_desc_k_sw128(smem_u32(sA + stage * TC_STAGE_BYTES));
-            const uint64_t bdesc = umma_desc_k_sw128(smem_u32(sW + kb * wbytes_kb));
+            const uint32_t a_addr = smem_u32(sA + stage * (SW ? stage_bytes : TC_STAGE_BYTES));
+            const uint64_t adesc = umma_desc_k_sw128(a_addr);
+            const uint64_t bdesc = umma_desc_k_sw128(SW ? a_addr + TC_STAGE_BYTES : smem_u32(sW + kb * wbytes_kb));
 #pragma unroll
             for (int k = 0; k < TC_BK / 16; ++k) {
               // advance 16 bf16 = 32 bytes along K inside the swizzle atom: +2 in the (addr >> 4) field
@@ -784,6 +792,24 @@ int pow2_floor_le(int v, int cap) {
   return r;
 }
 
+constexpr int TC_MAX_SMEM = 227 * 1024 - 1024 /*align*/ - 8192 /*barriers, bias, BatchNorm table, reduction scratch*/;
+
+// Weight placement of a lvae_conv2d_tc launch, from the shape alone: 0 = rejected, 1 = resident, 2 = streamed.  Resident
+// when the packed weights leave room for two 16 KB activation stages next to the largest output staging the shape can
+// use (the TMA-store epilogue's, bf16 output with N = 64 / 128); every shape a 64-filter model launches is resident.
+int tc_weight_plan(int Cin, int N, int ksize, int inputs, int H, int W, int out_f32) {
+  if (!(Cin % 64 == 0 && Cin >= 64 && Cin <= 256 && (ksize == 1 || ksize == 3) && N >= 1 && N <= 256)) return 0;
+  if (!(H > 0 && W > 0 && (W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W <= 128)) return 0;
+  const int n_kb = ksize * ksize * inputs * (Cin / 64);
+  if (n_kb > TC_MAX_KB) return 0;
+  const int Npad = (N + 15) / 16 * 16;
+  const int out_stage = (!out_f32 && N % 64 == 0 && N <= 128) ? Npad / 64 * TC_STAGE_BYTES : 0;
+  const int wbytes = ((n_kb * Npad * 128) + 1023) & ~1023;
+  if ((TC_MAX_SMEM - wbytes - out_stage) / TC_STAGE_BYTES >= 2) return 1;
+  if ((TC_MAX_SMEM - out_stage) / (TC_STAGE_BYTES + Npad * 128) >= 2) return 2;
+  return 0;
+}
+
 }  // namespace
 
 // x, x2: (B,H,W,Cin) bf16 NHWC, Cin a multiple of 64 (x2 optional: second input of a merge conv).
@@ -837,11 +863,6 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   LVAE_REQUIRE((W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W <= 128, "conv2d_tc: H and W must be powers of two (W <= 128)");
   LVAE_REQUIRE(!(y2 && res), "conv2d_tc: residual and split output are exclusive");
   LVAE_REQUIRE(!y2 || (nsplit % 16 == 0 && nsplit > 0 && nsplit < N), "conv2d_tc: nsplit must be a multiple of 16 inside (0, N)");
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    lvae_set_error("conv2d_tc: cuTensorMapEncodeTiled unavailable");
-    return LVAE_ERR_CUDA;
-  }
   TcParams p{};
   p.bias = bias; p.out_scale = out_scale; p.res = res; p.y = y; p.y2 = y2; p.nsplit = nsplit;
   p.M_total = B * H * W; p.H = H; p.W = W; p.N = N; p.Npad = (N + 15) / 16 * 16;
@@ -877,6 +898,10 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   const int cblocks = Cin / 64;
   p.n_kb = taps * inputs * cblocks;
   LVAE_REQUIRE(p.n_kb <= TC_MAX_KB, "conv2d_tc: too many k-blocks");
+  const int wplan = tc_weight_plan(Cin, N, ksize, inputs, H, W, out_f32);
+  LVAE_REQUIRE(wplan != 0, "conv2d_tc: weights leave no room for the activation pipeline");
+  const bool stream_w = wplan == 2;
+  LVAE_REQUIRE(!stream_w || !fuse, "conv2d_tc: fused epilogues need resident weights");
   int kb = 0;
   for (int t = 0; t < taps; ++t) {
     int ky = t / ksize, kx = t % ksize;
@@ -893,27 +918,33 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   p.tmem_cols = 32;
   while (p.tmem_cols < 2 * p.Npad) p.tmem_cols *= 2;
   LVAE_REQUIRE(p.tmem_cols <= 512, "conv2d_tc: accumulator does not fit TMEM");
-  const int max_smem = 227 * 1024 - 1024 /*align*/ - 8192 /*barriers, bias, BatchNorm table, reduction scratch*/;
-  const int wbytes = ((p.n_kb * p.Npad * 128) + 1023) & ~1023;
+  const int max_smem = TC_MAX_SMEM;
+  const int wbytes = stream_w ? 0 : ((p.n_kb * p.Npad * 128) + 1023) & ~1023;
   p.tma_store = (!out_f32 && N % 64 == 0 && N <= 128 && !res && (!y2 || nsplit % 64 == 0)) ? 1 : 0;
   const int out_stage = p.tma_store ? (p.Npad / 64 + (p.gate_x ? 1 : 0)) * TC_STAGE_BYTES : 0;
   LVAE_REQUIRE(!p.gate_x || p.tma_store, "conv2d_tc: the gated-residual epilogue needs the TMA-store path");
   LVAE_REQUIRE(!p.fold_gamma || p.tma_store, "conv2d_tc: the folded BatchNorm epilogue needs the TMA-store path");
   LVAE_REQUIRE(!(p.stats_acc || p.bnb_acc) || (p.tma_store && (N == 64 || p.gate_x) && !y2),
                "conv2d_tc: fused reductions need the TMA-store path (bf16 output, N == 64, no residual, no split)");
-  p.halo = (ksize == 3 && !x2 && Cin == 64 && W % 8 == 0 && H % 16 == 0 &&
+  p.halo = (!stream_w && ksize == 3 && !x2 && Cin == 64 && W % 8 == 0 && H % 16 == 0 &&
             (max_smem - wbytes - out_stage) / (18 * 16 * 128) >= 2) ? 1 : 0;
   p.stage_bytes = 18 * 16 * 128;
   p.tiles_x = W / 8;
   p.tiles_per_img = (W / 8) * (H / 16);
   set_shifts(p);
   LVAE_REQUIRE(!p.pre_gamma || p.halo, "conv2d_tc: the operand-path BatchNorm needs the halo-tile path (no shared memory left for two halo stages)");
-  int stages = (max_smem - wbytes - out_stage) / (p.halo ? p.stage_bytes : TC_STAGE_BYTES);
+  const int a_stage = p.halo ? p.stage_bytes : (stream_w ? TC_STAGE_BYTES + p.Npad * 128 : TC_STAGE_BYTES);
+  int stages = (max_smem - wbytes - out_stage) / a_stage;
   if (stages > 8) stages = 8;
   LVAE_REQUIRE(stages >= 2, "conv2d_tc: weights leave no room for the activation pipeline");
   p.n_stages = stages;
-  const size_t smem = 1024 + (size_t)wbytes + (size_t)stages * (p.halo ? p.stage_bytes : TC_STAGE_BYTES) + out_stage + 8192;
+  const size_t smem = 1024 + (size_t)wbytes + (size_t)stages * a_stage + out_stage + 8192;
 
+  EncodeTiledFn enc = get_encode();
+  if (!enc) {
+    lvae_set_error("conv2d_tc: cuTensorMapEncodeTiled unavailable");
+    return LVAE_ERR_CUDA;
+  }
   CUtensorMap tmA0, tmA1, tmW, tmY, tmY2;
   memset(&tmY, 0, sizeof(tmY));
   memset(&tmY2, 0, sizeof(tmY2));
@@ -964,6 +995,7 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<3, ACT_ELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<4, ACT_ELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<0, -1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e != cudaSuccess) { lvae_set_error("conv2d_tc: cannot raise dynamic smem: %s", cudaGetErrorString(e)); return LVAE_ERR_CUDA; }
     attr_smem = 227 * 1024;
   }
@@ -976,10 +1008,16 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   else if (p.stats_acc) lvae_launch(conv_tc_kernel<1>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.bnb_acc && p.bnb_act == ACT_ELU) lvae_launch(conv_tc_kernel<2, ACT_ELU>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.bnb_acc) lvae_launch(conv_tc_kernel<2>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
+  else if (stream_w) lvae_launch(conv_tc_kernel<0, -1, true>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else lvae_launch(conv_tc_kernel<0>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   LVAE_COUNT_LAUNCH();
   LVAE_CHECK_LAUNCH("conv2d_tc");
   return LVAE_OK;
+}
+
+// Pure-host query: how lvae_conv2d_tc would hold the weights of this shape (0 rejected, 1 resident, 2 streamed).
+LVAE_API int lvae_conv2d_tc_plan(int Cin, int N, int ksize, int two_inputs, int H, int W, int out_f32) {
+  return tc_weight_plan(Cin, N, ksize, two_inputs ? 2 : 1, H, W, out_f32);
 }
 
 // Stride-2 3x3 convolutions of 64 -> 64 channels on the same kernel (bf16 in / out, TMA-store epilogue).

@@ -34,6 +34,7 @@ struct WgParams {
   int tmem_cols;
   int tiles_per_cta;
   int dy_c0;                 // first dY channel of this launch (dY may be wider than N: split launches)
+  int x_c0;                  // first channel of the 64-channel X window (X, X2 may be wider than 64: split launches)
   // halo mode (3x3, one input, N = 64, W % 8 == 0, H % 16 == 0): pixel tiles are 16 rows x 8 columns and ONE TMA box of
   // 18 rows x 16 columns serves all nine taps (shifted MN-major descriptors, SBO = one 16-pixel image row = 2048 B)
   int halo, tiles_x, tiles_per_img;
@@ -165,7 +166,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         if (elect_one()) {
           uint8_t* stage = smem + st * WG_HALO_STAGE_BYTES;
           mbar_expect_tx(BAR(st), (uint32_t)WG_HALO_STAGE_BYTES);
-          tma_load_4d(smem_u32(stage), &tmX, BAR(st), 0, tx * 8 - 1, ty * 16 - 1, n0);
+          tma_load_4d(smem_u32(stage), &tmX, BAR(st), p.x_c0, tx * 8 - 1, ty * 16 - 1, n0);
           tma_load_4d(smem_u32(stage + WG_HALO_BYTES), &tmDY, BAR(st), p.dy_c0, tx * 8, ty * 16, n0);
         }
         __syncwarp();
@@ -199,7 +200,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
             for (int h = 0; h < 2; ++h) {
               int src = p.a_src[2 * pr + h];
               if (src < 2)
-                tma_load_4d(smem_u32(sPair + (ps * 2 + h) * WG_BLK_BYTES), src ? &tmX2 : &tmX, BAR(ps), 0,
+                tma_load_4d(smem_u32(sPair + (ps * 2 + h) * WG_BLK_BYTES), src ? &tmX2 : &tmX, BAR(ps), p.x_c0,
                             w0 * p.in_stride + p.a_dx[2 * pr + h], h0 * p.in_stride + p.a_dy[2 * pr + h], n0);
             }
           }
@@ -333,7 +334,9 @@ struct UnpackDesc {
   int n_pairs, N, taps, I_real, N_real, clear;
   int8_t kind[2 * WG_MAX_PAIRS];     // 0 tap block, 1 ones, 2 unused
   int8_t tap[2 * WG_MAX_PAIRS], ci0_blk[2 * WG_MAX_PAIRS];
-  int8_t pad_[2];
+  // X window of a split launch, in 64-channel blocks: the packed rows of input s hold dw input channels
+  // s * xC + x_c0 + [0, 64).  Both zero (xC = 64, x_c0 = 0) for the single-window launches the engine batches.
+  int8_t x_c0_blk, xC_blk;
 };
 static_assert(sizeof(UnpackDesc) == 80, "UnpackDesc layout is mirrored by engine.py");
 
@@ -348,6 +351,8 @@ __device__ __forceinline__ void unpack_body(const UnpackDesc& d, float (*tile)[9
   float* gp = const_cast<float*>(d.gp);
   const int n_items = d.n_pairs * 128 * (UNPACK_CO / 4);
   const bool clear = (d.clear & 1) != 0, overwrite = (d.clear & 2) != 0;
+  const bool windowed = d.x_c0_blk != 0 || d.xC_blk != 0;
+  const int xC = 64 * (d.xC_blk ? d.xC_blk : 1), x_c0 = 64 * d.x_c0_blk;
   // four independent 16-byte loads in flight per thread
   for (int base = threadIdx.x; base < n_items; base += 4 * blockDim.x) {
     float4 v[4];
@@ -366,8 +371,8 @@ __device__ __forceinline__ void unpack_body(const UnpackDesc& d, float (*tile)[9
       if (clear) *reinterpret_cast<float4*>(gp + (size_t)i * d.N + co0 + 4 * part) = make_float4(0.f, 0.f, 0.f, 0.f);
       const float vv[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
       if (kind == 0) {
-        const int cin = d.ci0_blk[blk] * 64 + ci;
-        if (cin < d.I_real) {
+        const int cin = d.ci0_blk[blk] * 64 + ci;                  // row of the packed gradient: input block, channel
+        if ((windowed ? d.ci0_blk[blk] * xC + x_c0 + ci : cin) < d.I_real) {
           const int o = cin * d.taps + d.tap[blk];
 #pragma unroll
           for (int e = 0; e < 4; ++e) tile[4 * part + e][o] = vv[e];
@@ -387,6 +392,22 @@ __device__ __forceinline__ void unpack_body(const UnpackDesc& d, float (*tile)[9
   const int nco = min(UNPACK_CO, d.N_real - co0);
   float* dst = d.dw + (size_t)co0 * run;
   const int total = nco * run;
+  if (windowed) {
+    // the tile holds 64 input channels per input, dw rows span all I_real of them: scatter each window into its place
+    int inputs = 0;
+    for (int b = 0; b < 2 * WG_MAX_PAIRS; ++b)
+      if (d.kind[b] == 0 && d.ci0_blk[b] + 1 > inputs) inputs = d.ci0_blk[b] + 1;
+    const int lrun = inputs * 64 * d.taps;                       // tile entries per output channel
+    for (int o = threadIdx.x; o < nco * lrun; o += blockDim.x) {
+      const int j = o / lrun, lo = o - j * lrun;
+      const int cl = lo / d.taps, t = lo - cl * d.taps;
+      const int cin = (cl >> 6) * xC + x_c0 + (cl & 63);
+      if (cin >= d.I_real) continue;
+      float* q = dst + (size_t)j * run + cin * d.taps + t;
+      *q = overwrite ? tile[j][lo] : *q + tile[j][lo];
+    }
+    return;
+  }
   if (overwrite) {
     for (int o = threadIdx.x; o < total; o += blockDim.x) dst[o] = tile[o / run][o % run];
   } else {
@@ -423,7 +444,7 @@ __global__ void __launch_bounds__(256) wgrad_unpack_one_kernel(const UnpackDesc 
 }
 
 void fill_unpack_desc(UnpackDesc* d, const float* gp, float* dw, float* dbias, int N, int ksize, int inputs, int I_real,
-                      int N_real, int clear) {
+                      int N_real, int clear, int xC = 64, int x_c0 = 0) {
   memset(d, 0, sizeof(*d));
   const int taps = ksize * ksize;
   int nblk = 0;
@@ -433,6 +454,10 @@ void fill_unpack_desc(UnpackDesc* d, const float* gp, float* dw, float* dbias, i
   d->kind[nblk] = 1; ++nblk;
   d->gp = gp; d->dw = dw; d->dbias = dbias; d->n_pairs = nblk / 2; d->N = N; d->taps = taps;
   d->I_real = I_real > 0 ? I_real : 64 * inputs; d->N_real = N_real > 0 ? N_real : N; d->clear = clear;
+  if (xC != 64 || x_c0 != 0) {
+    d->x_c0_blk = (int8_t)(x_c0 / 64); d->xC_blk = (int8_t)(xC / 64);
+    if (I_real <= 0) d->I_real = xC * inputs;
+  }
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -489,7 +514,7 @@ LVAE_API long long lvae_wgrad_tc_workspace(int B, int H, int W, int N, int ksize
 // Gp += wgrad.  x, x2: (B,H,W,64) bf16 (x2 optional); dY: (B,H,W,dyC) bf16 (dyC = 0 means N), already multiplied by any
 // Dropout2d mask; this launch uses its channels [dy_c0, dy_c0 + N), N in {64, 128}.  gp: lvae_wgrad_tc_packed_size floats.
 static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, float* gp, int B, int H, int W, int N,
-                             int ksize, int dyC, int dy_c0, int in_stride, cudaStream_t stream);
+                             int ksize, int dyC, int dy_c0, int in_stride, cudaStream_t stream, int xC = 64, int x_c0 = 0);
 
 LVAE_API int lvae_conv2d_wgrad_tc_acc(const void* x, const void* x2, const void* dy, float* gp, int B, int H, int W, int N,
                                       int ksize, int dyC, int dy_c0, cudaStream_t stream) {
@@ -506,13 +531,16 @@ LVAE_API int lvae_conv2d_wgrad_tc_s2_acc(const void* xs, const void* c, float* g
 }
 
 static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, float* gp, int B, int H, int W, int N,
-                             int ksize, int dyC, int dy_c0, int in_stride, cudaStream_t stream) {
+                             int ksize, int dyC, int dy_c0, int in_stride, cudaStream_t stream, int xC, int x_c0) {
   LVAE_REQUIRE(x && dy && gp, "conv2d_wgrad_tc: null pointer");
   LVAE_REQUIRE((N == 64 || N == 128) && (ksize == 1 || ksize == 3), "conv2d_wgrad_tc: N must be 64 or 128, ksize 1 or 3");
   LVAE_REQUIRE(B > 0 && H > 0 && W > 0 && (W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W <= 128,
                "conv2d_wgrad_tc: H and W must be powers of two (W <= 128), B positive");
   if (dyC <= 0) dyC = N;
   LVAE_REQUIRE(dy_c0 >= 0 && dy_c0 % 64 == 0 && dy_c0 + N <= dyC, "conv2d_wgrad_tc: bad dY channel window");
+  LVAE_REQUIRE(x_c0 >= 0, "conv2d_wgrad_tc: negative X channel window");
+  LVAE_REQUIRE(x_c0 % 64 == 0, "conv2d_wgrad_tc: X channel window not 64-aligned");
+  LVAE_REQUIRE(xC % 64 == 0 && xC <= 256 && x_c0 + 64 <= xC, "conv2d_wgrad_tc: X channel window past the %d input channels", xC);
   EncodeTiledFn enc = wg_get_encode();
   if (!enc) { lvae_set_error("conv2d_wgrad_tc: cuTensorMapEncodeTiled unavailable"); return LVAE_ERR_CUDA; }
   const int inputs = x2 ? 2 : 1, taps = ksize * ksize;
@@ -551,9 +579,10 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
   int bn = WG_TILE / (bw * bh);
   if (p.halo) { bw = 8; bh = 16; bn = 1; }
   CUtensorMap tmX, tmX2, tmDY, tmGp;
-  int r = p.halo ? make_act_map(enc, &tmX, x, B, H, W, 64, 16, 18, 1)
-                 : make_act_map(enc, &tmX, x, B, H * in_stride, W * in_stride, 64, bw, bh, bn, in_stride);
-  if (!r) r = make_act_map(enc, &tmX2, x2 ? x2 : x, B, H, W, 64, bw, bh, bn);
+  p.x_c0 = x_c0;
+  int r = p.halo ? make_act_map(enc, &tmX, x, B, H, W, xC, 16, 18, 1)
+                 : make_act_map(enc, &tmX, x, B, H * in_stride, W * in_stride, xC, bw, bh, bn, in_stride);
+  if (!r) r = make_act_map(enc, &tmX2, x2 ? x2 : x, B, H, W, xC, bw, bh, bn);
   p.dy_c0 = dy_c0;
   if (!r) r = make_act_map(enc, &tmDY, dy, B, H, W, dyC, bw, bh, bn);
   if (!r) {
@@ -620,20 +649,38 @@ LVAE_API int lvae_conv2d_wgrad_tc_s2(const void* xs, const void* c, float* dw, f
 
 // One-call form: dw (N_real, I_real, k, k) fp32 += wgrad, dbias [N_real] += column sums (or NULL).  x may carry zero-padded
 // channels beyond I_real (0 = none), dY beyond N_real (0 = none).  ws: lvae_wgrad_tc_workspace floats, overwritten.
+LVAE_API int lvae_conv2d_wgrad_tc_ex(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws,
+                                     int B, int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0,
+                                     int xC, int x_c0, cudaStream_t stream);
+
 LVAE_API int lvae_conv2d_wgrad_tc(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws,
                                   int B, int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0,
                                   cudaStream_t stream) {
+  return lvae_conv2d_wgrad_tc_ex(x, x2, dy, dw, dbias, ws, B, H, W, N, ksize, I_real, N_real, dyC, dy_c0, 0, 0, stream);
+}
+
+// The same over the 64-channel X window [x_c0, x_c0 + 64) of inputs with xC channels each (0 = 64): dw is (N_real, I_real,
+// k, k) with I_real = xC per input (0) or fewer, and this launch adds the window's columns of it.  The bias gradient comes
+// with every launch: pass dbias to exactly one launch per dY window.
+LVAE_API int lvae_conv2d_wgrad_tc_ex(const void* x, const void* x2, const void* dy, float* dw, float* dbias, float* ws,
+                                     int B, int H, int W, int N, int ksize, int I_real, int N_real, int dyC, int dy_c0,
+                                     int xC, int x_c0, cudaStream_t stream) {
   LVAE_REQUIRE(x && dy && dw && ws, "conv2d_wgrad_tc: null pointer");
   const long long n = lvae_wgrad_tc_packed_size(N, ksize, x2 != nullptr);
   LVAE_REQUIRE(n > 0, "conv2d_wgrad_tc: unsupported shape");
-  LVAE_REQUIRE(wgrad_real_ok(N, x2 ? 2 : 1, I_real, N_real),
-               "conv2d_wgrad_tc: I_real %d / N_real %d outside 0..%d / 0..%d", I_real, N_real, x2 ? 128 : 64, N);
+  if (xC <= 0) xC = 64;
+  const int inputs = x2 ? 2 : 1;
+  LVAE_REQUIRE(I_real >= 0 && I_real <= xC * inputs && N_real >= 0 && N_real <= N,
+               "conv2d_wgrad_tc: I_real %d / N_real %d outside 0..%d / 0..%d", I_real, N_real, xC * inputs, N);
+  LVAE_REQUIRE(x_c0 >= 0, "conv2d_wgrad_tc: negative X channel window");
+  LVAE_REQUIRE(x_c0 % 64 == 0, "conv2d_wgrad_tc: X channel window not 64-aligned");
+  LVAE_REQUIRE(xC % 64 == 0 && xC <= 256 && x_c0 + 64 <= xC, "conv2d_wgrad_tc: X channel window past the %d input channels", xC);
   cudaError_t e = cudaMemsetAsync(ws, 0, (size_t)n * 4, stream);
   if (e != cudaSuccess) { lvae_set_error("conv2d_wgrad_tc: memset failed: %s", cudaGetErrorString(e)); return LVAE_ERR_CUDA; }
-  int rc = lvae_conv2d_wgrad_tc_acc(x, x2, dy, ws, B, H, W, N, ksize, dyC, dy_c0, stream);
+  int rc = wgrad_tc_acc_impl(x, x2, dy, ws, B, H, W, N, ksize, dyC, dy_c0, 1, stream, xC, x_c0);
   if (rc) return rc;
   UnpackDesc d;
-  fill_unpack_desc(&d, ws, dw, dbias, N, ksize, x2 ? 2 : 1, I_real, N_real, 0);
+  fill_unpack_desc(&d, ws, dw, dbias, N, ksize, inputs, I_real, N_real, 0, xC, x_c0);
   lvae_launch(wgrad_unpack_one_kernel, dim3(cdiv(d.N_real, UNPACK_CO), 1), 256, 0, stream, d);
   LVAE_COUNT_LAUNCH();
   LVAE_CHECK_LAUNCH("wgrad_unpack");

@@ -377,6 +377,20 @@ def _pow2(v: int) -> bool:
     return v > 0 and (v & (v - 1)) == 0
 
 
+TC_REJECTED, TC_RESIDENT, TC_STREAMED = 0, 1, 2
+_tc_plans = {}
+
+
+def conv_tc_plan(cin: int, n: int, k: int, two_inputs: bool, h: int, w: int, out_f32: bool) -> int:
+    """How lvae_conv2d_tc holds the weights of this launch shape: TC_REJECTED, TC_RESIDENT or TC_STREAMED.  The library's
+    own rule (lvae_conv2d_tc_plan, the code the launch runs), asked once per shape."""
+    key = (cin, n, k, bool(two_inputs), h, w, bool(out_f32))
+    plan = _tc_plans.get(key)
+    if plan is None:
+        plan = _tc_plans[key] = int(_capi.lib().lvae_conv2d_tc_plan(*(int(v) for v in key)))
+    return plan
+
+
 class ConvSpec:
     """Static geometry + packed-weight caches of one conv module (Conv2d or ConvTranspose2d)."""
 
@@ -430,17 +444,18 @@ class ConvSpec:
         if not (_tc_enabled[0] and self.tc_shape and xn.dtype == torch.bfloat16 and self.cout <= 256):
             return False
         B, H, W, C = xn.shape
-        if not (_pow2(H) and _pow2(W) and W <= 128):
+        if not (_pow2(H) and _pow2(W) and W <= 128 and C % 64 == 0 and C <= 256):
             return False
-        if x2n is None:
-            return C % 64 == 0 and C <= 256
-        return C == 64 and x2n.shape[3] == 64
+        if x2n is not None and x2n.shape[3] != C:
+            return False
+        return conv_tc_plan(C, self.cout, self.k, x2n is not None, H, W, self.out_fp32) != TC_REJECTED
 
-    def tc_dgrad_ok(self, gyn) -> bool:
+    def tc_dgrad_ok(self, gyn, out_f32: bool = False) -> bool:
         if not (_tc_enabled[0] and self.tc_shape and self.cin <= 256):
             return False
         B, H, W, N = gyn.shape
-        return _pow2(H) and _pow2(W) and W <= 128 and N % 64 == 0 and N <= 256
+        return (_pow2(H) and _pow2(W) and W <= 128 and N % 64 == 0 and N <= 256
+                and conv_tc_plan(N, self.cin, self.k, False, H, W, out_f32) != TC_REJECTED)
 
 
 # Weight gradients depend only on saved activations and the output gradient, and nothing reads them before the
@@ -507,23 +522,32 @@ _wgrad_tc_fits = {}
 
 
 def wgrad_tc_plan(N: int, k: int, two_inputs: bool):
-    """Launches ((width, first dY channel), ...) of the tensor-core weight gradient of a stride-1 conv with N in {64, 128}
-    output channels, or () when the kernel cannot take it.  What fits is the library's own rule
-    (lvae_wgrad_tc_packed_size > 0); a 3x3 conv with N = 128 does not fit TMEM and runs as two launches over 64-channel
-    windows of dY.  PackedGradArena gives a packed gradient exactly to the single-launch shapes."""
+    """dY windows ((width, first dY channel), ...) of the tensor-core weight gradient of a stride-1 conv with N output
+    channels (a multiple of 64), or () when the kernel cannot take it.  What fits is the library's own rule
+    (lvae_wgrad_tc_packed_size > 0); a shape that does not fit TMEM runs over 128- or 64-channel windows of dY (a 3x3 conv
+    with N = 128: two launches).  PackedGradArena gives a packed gradient exactly to the single-launch shapes."""
     def fits(n):
         key = (n, k, bool(two_inputs))
         ok = _wgrad_tc_fits.get(key)
         if ok is None:
             ok = _wgrad_tc_fits[key] = int(_capi.lib().lvae_wgrad_tc_packed_size(n, k, int(bool(two_inputs)))) > 0
         return ok
-    if N not in (64, 128):
+    if N <= 0 or N % 64 or N > 256:
         return ()
-    if fits(N):
+    if N <= 128 and fits(N):
         return ((N, 0),)
-    if N == 128 and fits(64):
-        return ((64, 0), (64, 64))
+    for n in (128, 64):
+        if n < N and N % n == 0 and fits(n):
+            return tuple((n, c0) for c0 in range(0, N, n))
     return ()
+
+
+def wgrad_tc_windows(N: int, k: int, two_inputs: bool, xC: int):
+    """(first X channel, width, first dY channel) of every launch of the tensor-core weight gradient when each input has
+    xC > 64 channels: the dY windows of wgrad_tc_plan, once per 64-channel X window.  () when the kernel cannot take it."""
+    if xC % 64 or xC > 256:
+        return ()
+    return tuple((x0, n, c0) for x0 in range(0, xC, 64) for n, c0 in wgrad_tc_plan(N, k, two_inputs))
 
 
 def _tc_fusable(N, out_f32, res, nsplit=0) -> bool:
@@ -542,6 +566,9 @@ def _conv_tc(x, x2, wp, bias, out_scale, res, N, ksize, flip, out_f32, nsplit=0,
         y2 = torch.empty((B, H, W, N - nsplit), dtype=odt, device=x.device)
     else:
         y, y2 = torch.empty((B, H, W, N), dtype=odt, device=x.device), None
+    if conv_tc_plan(C, N, ksize, x2 is not None, H, W, out_f32) == TC_STREAMED:
+        key = "tc_dgrad_streamed" if flip else "tc_fwd_streamed"
+        stats[key] = stats.get(key, 0) + 1
     fuse = None
     gate_out = None
     if stats_acc is not None or bnb is not None or gate is not None or fold is not None:
@@ -641,8 +668,8 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
     _, Ho, Wo, N = gyn.shape
     gx = gx2 = gw = gb = None
     conv_backward_raw.last_fused = False
-    use_tc = xn.dtype == torch.bfloat16 and spec.tc_dgrad_ok(gyn)
     padded = x2n is None and C1 > spec.cin
+    use_tc = xn.dtype == torch.bfloat16 and spec.tc_dgrad_ok(gyn, padded)
     if padded and not use_tc:
         xn, C1, padded = xn[..., :spec.cin].contiguous(), spec.cin, False
     # stride-2 convs on the tensor cores: dgrad of Conv2d = "transposed" kind over the dy grid, dgrad of ConvTranspose2d =
@@ -693,10 +720,20 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
         gbbuf, bsunk = (None, True)
         if bias is not None and need_b:
             gbbuf, bsunk = _param_grad_buffer(bias)
-        plan = wgrad_tc_plan(N, spec.k, C2 > 0) if (use_tc and out_scale is None and C1 == 64 and C2 in (0, 64)
-                                                     and gyn.dtype == torch.bfloat16) else ()
+        tc_ok = use_tc and out_scale is None and gyn.dtype == torch.bfloat16 and C2 in (0, C1)
+        plan = wgrad_tc_plan(N, spec.k, C2 > 0) if (tc_ok and C1 == 64) else ()
+        wins = wgrad_tc_windows(N, spec.k, C2 > 0, C1) if (tc_ok and C1 > 64) else ()
         with _wgrad_stream(sunk and bsunk, (xn, x2n, gyn, out_scale)) as slot:
-            if plan:
+            if wins:
+                # wider inputs: one launch per (64-channel X window, dY window); the dY window's first X window adds the bias
+                stats["tc_wgrad"] += 1
+                stats["tc_wgrad_xwin"] = stats.get("tc_wgrad_xwin", 0) + 1
+                row = spec.cin * spec.k * spec.k * 4
+                for x0, n, c0 in wins:
+                    call("lvae_conv2d_wgrad_tc_ex", xn.data_ptr(), _p(x2n), gyn.data_ptr(), gwbuf.data_ptr() + c0 * row,
+                         None if (gbbuf is None or x0) else gbbuf.data_ptr() + c0 * 4,
+                         _wgrad_workspace(xn.device).data_ptr(), B, Hi, Wi, n, spec.k, 0, 0, N, c0, C1, x0, _stream())
+            elif plan:
                 stats["tc_wgrad"] += 1
                 gp = getattr(weight, "_lvae_gp", None) if (sunk and bsunk) else None
                 if gp is not None:
@@ -1533,7 +1570,7 @@ def dmol_loglik(l, x):
 
 
 class DmolHeadFn(Function):
-    """parameter_net conv (64 -> 100, 3x3) + mixture-of-logistics log-likelihood as ONE autograd node on the bf16
+    """parameter_net conv (64 or 128 -> 100, 3x3) + mixture-of-logistics log-likelihood as ONE autograd node on the bf16
     tensor-core path: the likelihood backward writes its gradient directly as the zero-padded bf16 operand
     (B,H,W,128) of the head conv's tcgen05 dgrad / wgrad (no fp32 round trip, no CUDA-core fallback for N = 100)."""
 
@@ -1580,19 +1617,34 @@ class DmolHeadFn(Function):
                 stats["tc_wgrad"] += 1
                 # five accumulator pairs x 128 columns would not fit TMEM: two launches over 64 output channels each
                 taps = spec.k * spec.k
-                for c0 in (0, 64):
-                    call("lvae_conv2d_wgrad_tc", hn.data_ptr(), None, dl.data_ptr(),
-                         gwbuf.data_ptr() + c0 * spec.cin * taps * 4, gbbuf.data_ptr() + c0 * 4,
-                         _wgrad_workspace(hn.device).data_ptr(), B, H, W, 64, spec.k, 0, min(64, spec.cout - c0), 128, c0,
-                         _stream())
+                if C == 64:
+                    for c0 in (0, 64):
+                        call("lvae_conv2d_wgrad_tc", hn.data_ptr(), None, dl.data_ptr(),
+                             gwbuf.data_ptr() + c0 * spec.cin * taps * 4, gbbuf.data_ptr() + c0 * 4,
+                             _wgrad_workspace(hn.device).data_ptr(), B, H, W, 64, spec.k, 0, min(64, spec.cout - c0), 128, c0,
+                             _stream())
+                else:
+                    # ... and, per dY window, one launch per 64-channel X window (the first adds the bias gradient)
+                    stats["tc_wgrad_xwin"] = stats.get("tc_wgrad_xwin", 0) + 1
+                    for x0 in range(0, C, 64):
+                        for c0 in (0, 64):
+                            call("lvae_conv2d_wgrad_tc_ex", hn.data_ptr(), None, dl.data_ptr(),
+                                 gwbuf.data_ptr() + c0 * spec.cin * taps * 4, None if x0 else gbbuf.data_ptr() + c0 * 4,
+                                 _wgrad_workspace(hn.device).data_ptr(), B, H, W, 64, spec.k, 0, min(64, spec.cout - c0), 128,
+                                 c0, C, x0, _stream())
             gw, gb = (None if sunk else gwbuf), (None if bsunk else gbbuf)
         return gh, gw, gb, None, None
 
 
 def dmol_head(h, conv, x):
     """Fused head when the tensor-core path applies; returns (ll, params) or None."""
-    hn_ok = h.dtype == torch.bfloat16 and conv.spec.cout == 100 and conv.spec.cin == 64 and _tc_enabled[0] \
+    hn_ok = h.dtype == torch.bfloat16 and conv.spec.cout == 100 and conv.spec.cin in (64, 128) and _tc_enabled[0] \
         and conv.spec.tc_shape and _pow2(h.shape[2]) and _pow2(h.shape[3]) and h.shape[3] <= 128
+    if hn_ok and conv.spec.cin != 64:
+        # wider input: the forward (N = 100, fp32 output) and the dgrad (N = cin) must be launches the library takes
+        H, W, k = h.shape[2], h.shape[3], conv.spec.k
+        hn_ok = (conv_tc_plan(conv.spec.cin, 100, k, False, H, W, True) != TC_REJECTED
+                 and conv_tc_plan(128, conv.spec.cin, k, False, H, W, False) != TC_REJECTED)
     if not hn_ok:
         return None
     return DmolHeadFn.apply(h, conv.weight, conv.bias, x, conv.spec)
