@@ -11,8 +11,7 @@
 // The MMA warp issues the 3x3 MMAs of tile i+1 before the gate MMAs of tile i, so the tensor pipe stays busy while the
 // epilogue warps stage tile i.  Same warp roles, descriptors, halo tiles and epilogue arithmetic as conv_tcgen05.cu
 // (which keeps serving every other convolution).
-#include "common.cuh"
-#include <cuda.h>
+#include "tcgen05.cuh"
 #include <string.h>
 
 namespace {
@@ -41,99 +40,6 @@ struct CgParams {
   int store_c2h;            // 1: c2 and h are stored (a backward pass will read them); 0: eval, only out leaves the SM
   long long* dbg;           // optional clock64 trace of CTA 0, 16 stamps per tile (lvae_conv_gate_tc_debug; normally null)
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {}
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* tm, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-               ::"l"(tm), "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* tm) {
-  asm volatile("prefetch.tensormap [%0];" ::"l"(tm) : "memory");
-}
-// K-major, 128B-swizzled operand tile: rows of 128 B, 8-row groups sbo bytes apart
-__device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t saddr, uint32_t sbo_bytes = 1024) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(sbo_bytes >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ uint32_t elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-template <int N> __device__ __forceinline__ void tmem_ldN_nowait(uint32_t taddr, uint32_t* r) {
-  if (N == 32) tmem_ld32_nowait(taddr, r);
-  else tmem_ld16_nowait(taddr, r);
-}
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // N (16 / 32) accumulator columns [c0, c0 + N) of this thread's row: + bias, * Dropout2d scale, packed to N / 8 16-byte bf16 chunks
 template <int N>
@@ -219,7 +125,7 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       mbar_init(BAR(B_A2F + g), 1);
       mbar_init(BAR(B_A2E + g), EW / G);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 0) {
     __syncwarp();
@@ -234,8 +140,7 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   for (int i = threadIdx.x; i < 192; i += CG_THREADS)
     sbias[i] = i < 64 ? (p.bias2 ? p.bias2[i] : 0.f) : (p.bias_g ? p.bias_g[i - 64] : 0.f);
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32(tmem_slot), tmem_cols);
   }
   tc_fence_before();
   __syncthreads();
@@ -279,8 +184,8 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     }
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
-    const uint32_t idesc3 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(64 >> 3) << 17) | ((uint32_t)(CG_BM >> 4) << 24);
-    const uint32_t idescg = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(CG_BM >> 4) << 24);
+    const uint32_t idesc3 = umma_idesc_bf16(CG_BM, 64, false, false);
+    const uint32_t idescg = umma_idesc_bf16(CG_BM, 128, false, false);
     const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
     mbar_wait(BAR(B_W), 0);
     tc_fence_after();
@@ -361,7 +266,7 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const int ew = warp - 2;
     float ra0 = 0.f, ra1 = 0.f, rb0 = 0.f, rb1 = 0.f;          // statistics of out, channels 2l and 2l+1
     const int rstep = p.halo ? p.W - 8 : 0;
-#define CG_EPI_BAR() asm volatile("bar.sync 1, %0;" ::"n"(32 * EW) : "memory")
+#define CG_EPI_BAR() named_bar_sync<1, 32 * EW>()
     if (fast) {
       // ---------------- eval mode (the IW evaluator's sample passes) ----------------
       // Group g = eight warps (TMEM lane quadrant x column half, 32 accumulator columns per thread) owns the CTA's tiles
@@ -376,7 +281,7 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const float* bg = sbias + 128 + 32 * half;
       const uint32_t lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16);
       auto group_bar = [&]() {
-        if (G == 2) asm volatile("bar.sync %0, 256;" ::"r"(1 + g) : "memory");
+        if (G == 2) asm volatile("bar.sync %0, 256;" ::"r"(1 + g) : "memory");   // runtime id (named_bar_sync takes immediates)
         else CG_EPI_BAR();
       };
       int it = 0;
@@ -419,13 +324,13 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(BAR(B_A1E + buf));           // the 3x3 accumulator is free for the tile after next
-          if (elected) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the group's previous `out` store has left the buffer
+          if (elected) bulk_wait_group_read<0>();   // the group's previous `out` store has left the buffer
           group_bar();
           uint8_t* blk = sStage + row * 128;
 #pragma unroll
           for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(blk + (((4 * half + q) ^ (row & 7)) << 4)) = pc[q];
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         group_bar();
         if (ew == 0 || ew == 8) CG_STAMP(3);
         if (elected) mbar_arrive(BAR(B_C2 + g));                  // the MMA warp may run the gate GEMM on the staged tile
@@ -471,15 +376,15 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
           for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(blk + (((4 * half + q) ^ (row & 7)) << 4)) = po[q];
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         group_bar();
         if (elected) {
           tma_store_4d(&tmOut, smem_u32(sStage), 0, c1, c2, c3);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
         }
         if (ew == 0 || ew == 8) CG_STAMP(6);
       }
-      if (elected) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+      if (elected) bulk_wait_group<0>();
     } else {
     int it = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
@@ -524,21 +429,21 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       if (lane == 0) mbar_arrive(BAR(B_A1E + buf));             // the 3x3 accumulator is free for the tile after next
       if (warp == 2) CG_STAMP(2);
       // every TMA store of the previous tile (c2, h, out) has finished reading the staging buffers
-      if (threadIdx.x == 64) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+      if (threadIdx.x == 64) bulk_wait_group_read<0>();
       CG_EPI_BAR();
       {
         uint8_t* blk = sC2 + row * 128;
 #pragma unroll
         for (int q = 0; q < NQ; ++q) *reinterpret_cast<uint4*>(blk + (((NQ * part + q) ^ (row & 7)) << 4)) = pc[q];
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to TMA and tcgen05.mma
+      fence_proxy_async();   // generic writes -> visible to TMA and tcgen05.mma
       CG_EPI_BAR();
       if (warp == 2) CG_STAMP(3);
       if (threadIdx.x == 64) {
         mbar_arrive(BAR(B_C2));                                  // the MMA warp may run the gate GEMM on the staged tile
         if (p.store_c2h) {
           tma_store_4d(&tmC2, smem_u32(sC2), 0, c1, c2, c3);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
         }
       }
       // residual rows for the gate pass: in flight while the gate GEMM runs
@@ -571,15 +476,15 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(BAR(B_A2E));                    // acc2 is free for the next tile's gate GEMM
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       CG_EPI_BAR();
       if (threadIdx.x == 64) {
         if (p.store_c2h) {
           tma_store_4d(&tmH, smem_u32(sH), 0, c1, c2, c3);
           tma_store_4d(&tmH, smem_u32(sH + CG_TILE_BYTES), 64, c1, c2, c3);
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
           // the c2 store (the older group) must have finished reading sC2 before the gate pass overwrites it with `out`
-          asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+          bulk_wait_group_read<1>();
         }
       }
       CG_EPI_BAR();
@@ -607,11 +512,11 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
       }
       if (warp == 2) CG_STAMP(5);
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       CG_EPI_BAR();
       if (threadIdx.x == 64) {
         tma_store_4d(&tmOut, smem_u32(sC2), 0, c1, c2, c3);
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        bulk_commit_group();
       }
       if (warp == 2) CG_STAMP(6);
     }
@@ -642,33 +547,10 @@ conv_gate_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     }
 #undef CG_EPI_BAR
   }
-  if (threadIdx.x == 64) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+  if (threadIdx.x == 64) bulk_wait_group<0>();
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_cg() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
-}
-
-int pow2_floor_le_cg(int v, int cap) {
-  int r = 1;
-  while (r * 2 <= v && r * 2 <= cap) r *= 2;
-  return r;
+  if (warp == 1) tmem_dealloc(tmem_base, tmem_cols);
 }
 
 long long* g_cg_dbg = nullptr;
@@ -688,7 +570,7 @@ LVAE_API int lvae_conv_gate_tc(const void* a2, const void* w2p, const float* bia
   LVAE_REQUIRE((c2 == nullptr) == (h == nullptr), "conv_gate_tc: c2 and h are stored together or not at all");
   LVAE_REQUIRE(B > 0 && (W & (W - 1)) == 0 && (H & (H - 1)) == 0 && W >= 1 && W <= 128 && H >= 1,
                "conv_gate_tc: H and W must be powers of two (W <= 128)");
-  EncodeTiledFn enc = get_encode_cg();
+  EncodeTiledFn enc = get_encode();
   if (!enc) { lvae_set_error("conv_gate_tc: cuTensorMapEncodeTiled unavailable"); return LVAE_ERR_CUDA; }
   CgParams p{};
   p.bias2 = bias2; p.scale2 = scale2; p.bias_g = bias_g; p.x_res = (const __nv_bfloat16*)x_res; p.stats_acc = stats_acc;
@@ -700,11 +582,10 @@ LVAE_API int lvae_conv_gate_tc(const void* a2, const void* w2p, const float* bia
   p.stage_bytes = p.halo ? CG_HALO_BYTES : CG_TILE_BYTES;
   p.tiles_x = W / 8;
   p.tiles_per_img = (W / 8) * (H / 16);
-  auto lg2 = [](int v) { int l = 0; while ((1 << l) < v) ++l; return l; };
-  p.lg_w = lg2(W); p.lg_hw = lg2(H * W); p.lg_tx = lg2(p.tiles_x > 0 ? p.tiles_x : 1);
-  p.lg_tpi = lg2(p.tiles_per_img > 0 ? p.tiles_per_img : 1);
+  p.lg_w = lg2_ceil(W); p.lg_hw = lg2_ceil(H * W); p.lg_tx = lg2_ceil(p.tiles_x > 0 ? p.tiles_x : 1);
+  p.lg_tpi = lg2_ceil(p.tiles_per_img > 0 ? p.tiles_per_img : 1);
   p.bw = W;
-  p.bh = pow2_floor_le_cg(H, CG_BM / p.bw);
+  p.bh = pow2_floor_le(H, CG_BM / p.bw);
   p.bn = CG_BM / (p.bw * p.bh);
   const int fixed = 1024 + CG_TAPS * 64 * 128 + 128 * 128 + 3 * CG_TILE_BYTES + 8192;
   int stages = (227 * 1024 - fixed) / p.stage_bytes;
@@ -716,37 +597,17 @@ LVAE_API int lvae_conv_gate_tc(const void* a2, const void* w2p, const float* bia
   CUtensorMap tmA, tmW2, tmWg, tmC2, tmH, tmOut;
   memset(&tmC2, 0, sizeof(tmC2));
   memset(&tmH, 0, sizeof(tmH));
-  const cuuint32_t one[4] = {1, 1, 1, 1};
-  auto enc_act = [&](CUtensorMap* tm, void* ptr, int ncols, bool load) -> CUresult {
-    cuuint64_t gdim[4] = {(cuuint64_t)ncols, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-    cuuint64_t gstr[3] = {(cuuint64_t)ncols * 2, (cuuint64_t)W * ncols * 2, (cuuint64_t)H * W * ncols * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)p.bw, (cuuint32_t)p.bh, (cuuint32_t)p.bn};
-    if (p.halo) {
-      if (load) { box[1] = 16; box[2] = 18; box[3] = 1; }
-      else { box[1] = 8; box[2] = 16; box[3] = 1; }
-    }
-    return enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, gdim, gstr, box, one, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  };
-  CUresult r = enc_act(&tmA, (void*)a2, 64, true);
-  if (r == CUDA_SUCCESS) r = enc_act(&tmOut, out, 64, false);
-  if (r == CUDA_SUCCESS && c2) r = enc_act(&tmC2, c2, 64, false);
-  if (r == CUDA_SUCCESS && h) r = enc_act(&tmH, h, 128, false);
+  // halo mode: a2 is loaded in boxes of 18 rows x 16 columns around each 16 x 8-pixel tile, the outputs are stored per tile
+  const int lbw = p.halo ? 16 : p.bw, lbh = p.halo ? 18 : p.bh;
+  const int sbw = p.halo ? 8 : p.bw, sbh = p.halo ? 16 : p.bh, bn = p.halo ? 1 : p.bn;
+  CUresult r = make_act_map(enc, &tmA, a2, B, H, W, 64, lbw, lbh, bn);
+  if (r == CUDA_SUCCESS) r = make_act_map(enc, &tmOut, out, B, H, W, 64, sbw, sbh, bn);
+  if (r == CUDA_SUCCESS && c2) r = make_act_map(enc, &tmC2, c2, B, H, W, 64, sbw, sbh, bn);
+  if (r == CUDA_SUCCESS && h) r = make_act_map(enc, &tmH, h, B, H, W, 128, sbw, sbh, bn);
   if (r != CUDA_SUCCESS) { lvae_set_error("conv_gate_tc: tensor map (activation) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
-  {
-    cuuint64_t wstr[1] = {128};
-    cuuint32_t westr[2] = {1, 1};
-    cuuint64_t wdim2[2] = {64, (cuuint64_t)CG_TAPS * 64};
-    cuuint32_t wbox2[2] = {64, 64};
-    r = enc(&tmW2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)w2p, wdim2, wstr, wbox2, westr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    cuuint64_t wdimg[2] = {64, 128};
-    cuuint32_t wboxg[2] = {64, 128};
-    if (r == CUDA_SUCCESS)
-      r = enc(&tmWg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)wgp, wdimg, wstr, wboxg, westr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { lvae_set_error("conv_gate_tc: tensor map (weights) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
-  }
+  r = make_weight_map(enc, &tmW2, w2p, CG_TAPS * 64, 64);
+  if (r == CUDA_SUCCESS) r = make_weight_map(enc, &tmWg, wgp, 128, 128);
+  if (r != CUDA_SUCCESS) { lvae_set_error("conv_gate_tc: tensor map (weights) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
   static bool attr = false;
   if (!attr) {
     cudaError_t e = cudaFuncSetAttribute(conv_gate_tc_kernel<ACT_ELU, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024));

@@ -20,8 +20,7 @@
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + single-thread MMA
 // issuer, warps 2..9 = epilogue (TMEM lane quadrant = warp_id % 4, two warps per quadrant split the columns).  The accumulator is double
 // buffered in TMEM so the epilogue of tile i overlaps the MMAs of tile i+1.
-#include "common.cuh"
-#include <cuda.h>
+#include "tcgen05.cuh"
 #include <string.h>
 #include <mutex>
 
@@ -83,110 +82,6 @@ struct TcParams {
   int in_stride, use_wblk;
   int8_t wblk[TC_MAX_KB];
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {}
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* tm, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-               ::"l"(tm), "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* tm) {
-  asm volatile("prefetch.tensormap [%0];" ::"l"(tm) : "memory");
-}
-// K-major, 128B-swizzled operand tile: rows of 128 B, 8-row groups 1024 B apart (SBO), version 1
-__device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);          // start address
-  d |= (uint64_t)1 << 16;                            // LBO (unused for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                  // SBO
-  d |= (uint64_t)1 << 46;                            // descriptor version (Blackwell)
-  d |= (uint64_t)2 << 61;                            // SWIZZLE_128B
-  return d;
-}
-// same, with the 8-row groups sbo bytes apart and a start address that is only 128-byte aligned.  The base-offset field
-// stays zero: the hardware swizzle is a function of the absolute shared-memory address
-__device__ __forceinline__ uint64_t umma_desc_k_sw128_shifted(uint32_t saddr, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(sbo_bytes >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// one elected lane of a fully converged warp (lets ptxas keep the MMA operands in uniform registers instead of
-// wrapping every tcgen05.mma in a per-lane broadcast loop)
-__device__ __forceinline__ uint32_t elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // Epilogue for 16 accumulator columns [c0, c0+16) of one output row: bias (shared memory), Dropout2d scale,
 // residual, conversion, vectorised store.  All global reads go through the read-only path so that the
@@ -313,7 +208,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     mbar_init(BAR(2 * S + 3), 8);                  // one arrive per epilogue warp
     mbar_init(BAR(2 * S + 4), 8);
     if (FUSE == 4) for (int i = 0; i < S; ++i) mbar_init(BAR(2 * S + 5 + i), 5);     // one arrive per transform warp
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   if (warp == 0 && !SW) {
     __syncwarp();
@@ -342,8 +237,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     for (int i = threadIdx.x; i < p.Npad; i += TC_THREADS) sbias[i] = (p.bias && i < p.N) ? p.bias[i] : 0.f;
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(p.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   }
   tc_fence_before();
   __syncthreads();
@@ -398,8 +292,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     // The whole warp runs the loop (converged); one elected lane issues tcgen05.mma / tcgen05.commit, so ptxas keeps
     // descriptors and the TMEM address in uniform registers.
     {
-      // instruction descriptor: D fp32, A/B bf16, both K-major, M = 128, N = Npad
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.Npad >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
+      const uint32_t idesc = umma_idesc_bf16(TC_BM, p.Npad, false, false);      // both operands K-major
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       if (!SW) mbar_wait(BAR(2 * S), 0);
       tc_fence_after();
@@ -422,7 +315,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             for (int kb = 0; kb < p.n_kb; ++kb) {
               // tap (dy,dx): the tile's first pixel sits at halo row 1+dy, halo column 1+dx; rows are 16 pixels (2048 B)
               const uint32_t a_start = a_base + (uint32_t)(((1 + p.dy[kb]) * 16 + (1 + p.dx[kb])) * 128);
-              const uint64_t adesc = umma_desc_k_sw128_shifted(a_start, 2048);
+              const uint64_t adesc = umma_desc_k_sw128(a_start, 2048);
               const uint64_t bdesc = umma_desc_k_sw128(smem_u32(sW + kb * wbytes_kb));
 #pragma unroll
               for (int k = 0; k < TC_BK / 16; ++k) {
@@ -496,7 +389,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             *ptr = make_uint4(w[0], w[1], w[2], w[3]);
           }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to tcgen05.mma
+        fence_proxy_async();   // generic writes -> visible to tcgen05.mma
         __syncwarp();
         if (lane == 0) mbar_arrive(BAR(2 * S + 5 + stage));
         if (++stage == S) { stage = 0; phase ^= 1; }
@@ -608,8 +501,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
         if (lane == 0) mbar_arrive(BAR(2 * S + 3 + buf));          // accumulator free again: next-but-one tile may start
         if (FUSE == 3) load_xq(rbase);                               // residual input rows (in flight across the staging barriers)
         // the previous tile's TMA store must have finished reading the staging buffer
-        if (threadIdx.x == 64) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        asm volatile("bar.sync 1, 256;" ::: "memory");
+        if (threadIdx.x == 64) bulk_wait_group_read<0>();
+        named_bar_sync<1, 256>();
 #pragma unroll
         for (int nch = 0; nch < NCH; ++nch) {
           const int c0 = 32 * half + 64 * nch;
@@ -621,8 +514,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             *reinterpret_cast<uint4*>(blk + ((chunk ^ (row & 7)) << 4)) = packed[nch][q];
           }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("bar.sync 1, 256;" ::: "memory");
+        fence_proxy_async();
+        named_bar_sync<1, 256>();
         if (threadIdx.x == 64) {
           int c1, c2, c3;
           if (p.halo) {
@@ -639,7 +532,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             const bool second = p.y2 != nullptr && j * 64 >= p.nsplit;
             tma_store_4d(second ? &tmY2 : &tmY, smem_u32(sOut + j * TC_STAGE_BYTES), second ? j * 64 - p.nsplit : j * 64, c1, c2, c3);
           }
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          bulk_commit_group();
         }
         if (FUSE == 3) {
           // gate pass over the staged h tile (a = block 0, gate = block 1; values as stored): out -> third staging block
@@ -665,8 +558,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
               rb0 = fmaf(q0, q0, rb0); rb1 = fmaf(q1, q1, rb1);
             }
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          asm volatile("bar.sync 1, 256;" ::: "memory");
+          fence_proxy_async();
+          named_bar_sync<1, 256>();
           if (threadIdx.x == 64) {
             int c1, c2, c3;
             if (p.halo) {
@@ -680,7 +573,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
               c2 = rem >> p.lg_w; c1 = rem & (p.W - 1);
             }
             tma_store_4d(&tmY2, smem_u32(sGate), 0, c1, c2, c3);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            bulk_commit_group();
           }
         } else if (FUSE == 1 || FUSE == 2) {
           // second pass over the staged tile (values as stored, bf16-rounded); the TMA store only reads it concurrently
@@ -741,7 +634,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
       // combine the eight row groups per channel: one double atomic per channel and statistic per CTA
       sred[(0 * 8 + ew) * 64 + 2 * lane] = ra0; sred[(0 * 8 + ew) * 64 + 2 * lane + 1] = ra1;
       sred[(1 * 8 + ew) * 64 + 2 * lane] = rb0; sred[(1 * 8 + ew) * 64 + 2 * lane + 1] = rb1;
-      asm volatile("bar.sync 1, 256;" ::: "memory");
+      named_bar_sync<1, 256>();
       const int t = threadIdx.x - 64;                              // 0..127 -> (statistic, channel)
       if (t < 128) {
         const int st = t >> 6, c = t & 63;
@@ -753,43 +646,17 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
       }
     }
   }
-  if (p.tma_store && threadIdx.x == 64) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+  if (p.tma_store && threadIdx.x == 64) bulk_wait_group<0>();
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
+  if (warp == 1) tmem_dealloc(tmem_base, p.tmem_cols);
 }
 
 long long* g_tc_dbg = nullptr;
 
-int lg2_ceil(int v) {
-  int l = 0;
-  while ((1 << l) < v) ++l;
-  return l;
-}
 void set_shifts(TcParams& p) {
   p.lg_w = lg2_ceil(p.W); p.lg_hw = lg2_ceil(p.H * p.W);
   p.lg_tx = lg2_ceil(p.tiles_x > 0 ? p.tiles_x : 1); p.lg_tpi = lg2_ceil(p.tiles_per_img > 0 ? p.tiles_per_img : 1);
-}
-
-int pow2_floor_le(int v, int cap) {
-  int r = 1;
-  while (r * 2 <= v && r * 2 <= cap) r *= 2;
-  return r;
 }
 
 constexpr int TC_MAX_SMEM = 227 * 1024 - 1024 /*align*/ - 8192 /*barriers, bias, BatchNorm table, reduction scratch*/;
@@ -953,35 +820,21 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
     void* const gate_out = (fuse && fuse->gate_out) ? fuse->gate_out : nullptr;
     for (int which = (gate_out && p.gate_skip_h) ? 1 : 0; which < ((y2 || gate_out) ? 2 : 1); ++which) {
       const int ncols = gate_out ? (which ? 64 : N) : (y2 ? (which ? N - nsplit : nsplit) : N);
-      cuuint64_t gdim[4] = {(cuuint64_t)ncols, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-      cuuint64_t gstr[3] = {(cuuint64_t)ncols * 2, (cuuint64_t)W * ncols * 2, (cuuint64_t)H * W * ncols * 2};
-      cuuint32_t box[4] = {64, (cuuint32_t)p.bw, (cuuint32_t)p.bh, (cuuint32_t)p.bn};
-      if (p.halo) { box[1] = 8; box[2] = 16; box[3] = 1; }
-      cuuint32_t estr[4] = {1, 1, 1, 1};
-      CUresult r = enc(which ? &tmY2 : &tmY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, which ? (gate_out ? gate_out : y2) : y, gdim, gstr, box, estr,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      CUtensorMap* tm = which ? &tmY2 : &tmY;
+      void* const dst = which ? (gate_out ? gate_out : y2) : y;
+      CUresult r = p.halo ? make_act_map(enc, tm, dst, B, H, W, ncols, 8, 16, 1)
+                          : make_act_map(enc, tm, dst, B, H, W, ncols, p.bw, p.bh, p.bn);
       if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc: tensor map (y) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
     }
   }
   {
-    cuuint64_t gdim[4] = {(cuuint64_t)Cin, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-    cuuint64_t gstr[3] = {(cuuint64_t)Cin * 2, (cuuint64_t)W * Cin * 2, (cuuint64_t)H * W * Cin * 2};
-    cuuint32_t box[4] = {64, (cuuint32_t)p.bw, (cuuint32_t)p.bh, (cuuint32_t)p.bn};
-    if (p.halo) { box[1] = 16; box[2] = 18; box[3] = 1; }
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(&tmA0, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)x, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    // activation maps: the tile's pixel box, or in halo mode 18 rows x 16 columns around the 16 x 8-pixel tile
+    const int bw = p.halo ? 16 : p.bw, bh = p.halo ? 18 : p.bh, bn = p.halo ? 1 : p.bn;
+    CUresult r = make_act_map(enc, &tmA0, x, B, H, W, Cin, bw, bh, bn);
     if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc: tensor map (x) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
-    r = enc(&tmA1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)(x2 ? x2 : x), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    r = make_act_map(enc, &tmA1, x2 ? x2 : x, B, H, W, Cin, bw, bh, bn);
     if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc: tensor map (x2) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
-    cuuint64_t wdim[2] = {64, (cuuint64_t)p.n_kb * p.Npad};
-    cuuint64_t wstr[1] = {128};
-    cuuint32_t wbox[2] = {64, (cuuint32_t)p.Npad};
-    cuuint32_t westr[2] = {1, 1};
-    r = enc(&tmW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)wp, wdim, wstr, wbox, westr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    r = make_weight_map(enc, &tmW, wp, p.n_kb * p.Npad, p.Npad);
     if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc: tensor map (w) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
   }
   static size_t attr_smem = 0;
@@ -1083,12 +936,7 @@ LVAE_API int lvae_conv2d_tc_s2(const void* x, const void* wp, const float* bias,
       // input: for kind 0 the (bigger) input grid is traversed with element stride 2, so a box of 2*bw x 2*bh input
       // pixels delivers the bw x bh pixels one filter tap needs for a tile of output pixels
       const int Hi = kind == 0 ? Hb : Hg, Wi = kind == 0 ? Wb : Wg, st = kind == 0 ? 2 : 1;
-      cuuint64_t gdim[4] = {(cuuint64_t)Cin, (cuuint64_t)Wi, (cuuint64_t)Hi, (cuuint64_t)B};
-      cuuint64_t gstr[3] = {(cuuint64_t)Cin * 2, (cuuint64_t)Wi * Cin * 2, (cuuint64_t)Hi * Wi * Cin * 2};
-      cuuint32_t box[4] = {64, (cuuint32_t)(p.bw * st), (cuuint32_t)(p.bh * st), (cuuint32_t)p.bn};
-      cuuint32_t estr[4] = {1, (cuuint32_t)st, (cuuint32_t)st, 1};
-      CUresult r = enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)x, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      CUresult r = make_act_map(enc, &tmA, x, B, Hi, Wi, Cin, p.bw, p.bh, p.bn, st);
       if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc_s2: tensor map (x) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
       // output: kind 0 the plain (B,Hg,Wg,N) tensor; kind 1 the parity class (py,px) of the (B,2Hg,2Wg,N) tensor
       const size_t Wo = kind == 0 ? Wg : Wb, Ho = kind == 0 ? Hg : Hb, step = kind == 0 ? 1 : 2;
@@ -1100,12 +948,7 @@ LVAE_API int lvae_conv2d_tc_s2(const void* x, const void* wp, const float* bias,
       r = enc(&tmY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)ybase, odim, ostr, obox, one, CU_TENSOR_MAP_INTERLEAVE_NONE,
               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
       if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc_s2: tensor map (y) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
-      cuuint64_t wdim[2] = {64, (cuuint64_t)9 * p.Npad};
-      cuuint64_t wstr[1] = {128};
-      cuuint32_t wbox[2] = {64, (cuuint32_t)p.Npad};
-      cuuint32_t westr[2] = {1, 1};
-      r = enc(&tmW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)wp, wdim, wstr, wbox, westr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      r = make_weight_map(enc, &tmW, wp, 9 * p.Npad, p.Npad);
       if (r != CUDA_SUCCESS) { lvae_set_error("conv2d_tc_s2: tensor map (w) encode failed: %d", (int)r); return LVAE_ERR_CUDA; }
     }
     const int n_tiles = (p.M_total + TC_BM - 1) / TC_BM;

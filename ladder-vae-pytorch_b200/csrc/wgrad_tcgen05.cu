@@ -11,8 +11,7 @@
 // Gp[(pair, row)][co] with TMA reduce-stores (cp.reduce.async.bulk.tensor ... .add: the additions happen in L2, there is
 // no per-CTA workspace and no reduction pass).  lvae_wgrad_unpack[_batched] re-lays Gp into the (O, I, kh, kw) gradient.
 // Shifted 4-D TMA boxes implement im2col, out-of-bounds zero fill implements the padding.
-#include "common.cuh"
-#include <cuda.h>
+#include "tcgen05.cuh"
 #include <string.h>
 
 namespace {
@@ -46,74 +45,6 @@ struct WgParams {
   int8_t a_src[2 * WG_MAX_PAIRS], a_dx[2 * WG_MAX_PAIRS], a_dy[2 * WG_MAX_PAIRS];
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {}
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-// MN-major, 128B-swizzled operand: 64 MN elements per 128-byte row, 8 K-rows per 1024-byte atom (SBO),
-// next block of 64 MN elements LBO bytes further.
-__device__ __forceinline__ uint64_t umma_desc_mn_sw128(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes = 1024) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFF) >> 4);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)(sbo_bytes >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ uint32_t elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
 __global__ void __launch_bounds__(WG_THREADS_TC, 1)
 wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmX2,
                 const __grid_constant__ CUtensorMap tmDY, const __grid_constant__ CUtensorMap tmGp, const WgParams p) {
@@ -137,14 +68,13 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < 13; ++i) mbar_init(BAR(i), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   // all-ones tile (any swizzle of a constant tile is the same tile)
   for (int i = threadIdx.x; i < WG_BLK_BYTES / 4; i += WG_THREADS_TC) ((uint32_t*)sOnes)[i] = 0x3F803F80u;
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the tensor core (async proxy)
+  fence_proxy_async();                                          // generic-proxy writes -> visible to the tensor core (async proxy)
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(p.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(smem_u32(tmem_slot), p.tmem_cols);
   }
   tc_fence_before();
   __syncthreads();
@@ -213,9 +143,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     {
       // ===================== MMA issuer (whole warp loops, one elected lane issues) =====================
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      // D fp32, A/B bf16, both MN-major, M = 128, N = 64 * n_bblk
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
-                             ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      const uint32_t idesc = umma_idesc_bf16(128, N, true, true);      // both operands MN-major
       int ps = 0, bs = 0;
       uint32_t pph = 0, bph = 0;
       if (p.halo) {
@@ -300,29 +228,27 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         for (int c0 = 0; c0 < N; c0 += 32, ++nbuf) {
           uint8_t* stg = smem + (nbuf & 1) * WG_BLK_BYTES;
           uint32_t r[32];
-          tmem_ld32(taddr + (uint32_t)c0, r);
-          if (leader) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the store two tiles back has read its buffer
-          asm volatile("bar.sync 1, 128;" ::: "memory");
+          tmem_ld32_nowait(taddr + (uint32_t)c0, r);
+          tmem_wait_ld();
+          if (leader) bulk_wait_group_read<1>();   // the store two tiles back has read its buffer
+          named_bar_sync<1, 128>();
 #pragma unroll
           for (int q = 0; q < 8; ++q)
             *reinterpret_cast<uint4*>(stg + row * 128 + ((q ^ (row & 7)) << 4)) = make_uint4(r[4 * q], r[4 * q + 1], r[4 * q + 2], r[4 * q + 3]);
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          asm volatile("bar.sync 1, 128;" ::: "memory");
+          fence_proxy_async();
+          named_bar_sync<1, 128>();
           if (leader) {
-            asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];"
-                         ::"l"(&tmGp), "r"(smem_u32(stg)), "r"(c0), "r"(pr * 128) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            tma_reduce_add_2d(&tmGp, smem_u32(stg), c0, pr * 128);
+            bulk_commit_group();
           }
         }
       }
-      if (leader) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+      if (leader) bulk_wait_group<0>();
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, p.tmem_cols);
 }
 
 // Packed gradient Gp -> torch-layout gradient.  Block blk (= pair*2 + half) of Gp holds 64 rows x N columns of kind
@@ -460,29 +386,6 @@ void fill_unpack_desc(UnpackDesc* d, const float* gp, float* dw, float* dbias, i
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn wg_get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)ptr;
-  }
-  return fn;
-}
-
-int make_act_map(EncodeTiledFn enc, CUtensorMap* tm, const void* ptr, int B, int H, int W, int C, int bw, int bh, int bn, int st = 1) {
-  cuuint64_t gdim[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  cuuint64_t gstr[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)(bw * st), (cuuint32_t)(bh * st), (cuuint32_t)bn};
-  cuuint32_t estr[4] = {1, (cuuint32_t)st, (cuuint32_t)st, 1};
-  return (int)enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, (void*)ptr, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-}
-
 }  // namespace
 
 static bool wgrad_shape_ok(int N, int ksize, int inputs) {
@@ -541,7 +444,7 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
   LVAE_REQUIRE(x_c0 >= 0, "conv2d_wgrad_tc: negative X channel window");
   LVAE_REQUIRE(x_c0 % 64 == 0, "conv2d_wgrad_tc: X channel window not 64-aligned");
   LVAE_REQUIRE(xC % 64 == 0 && xC <= 256 && x_c0 + 64 <= xC, "conv2d_wgrad_tc: X channel window past the %d input channels", xC);
-  EncodeTiledFn enc = wg_get_encode();
+  EncodeTiledFn enc = get_encode();
   if (!enc) { lvae_set_error("conv2d_wgrad_tc: cuTensorMapEncodeTiled unavailable"); return LVAE_ERR_CUDA; }
   const int inputs = x2 ? 2 : 1, taps = ksize * ksize;
   LVAE_REQUIRE(wgrad_shape_ok(N, ksize, inputs), "conv2d_wgrad_tc: too many operand blocks (3x3 over two inputs is not supported)");
@@ -574,8 +477,7 @@ static int wgrad_tc_acc_impl(const void* x, const void* x2, const void* dy, floa
   p.tiles_per_cta = (n_tiles + grid - 1) / grid;
   grid = (n_tiles + p.tiles_per_cta - 1) / p.tiles_per_cta;
   int bw = W;
-  int bh = 1;
-  while (bh * 2 <= H && bh * 2 * bw <= WG_TILE) bh *= 2;
+  int bh = pow2_floor_le(H, WG_TILE / bw);
   int bn = WG_TILE / (bw * bh);
   if (p.halo) { bw = 8; bh = 16; bn = 1; }
   CUtensorMap tmX, tmX2, tmDY, tmGp;
