@@ -101,8 +101,11 @@ int lvae_wgrad_unpack_desc_size(void);
 int lvae_wgrad_unpack_desc(void* desc_host, const float* gp, float* dw, float* dbias, int N, int ksize, int two_inputs,
                            int I_real, int N_real, int clear);
 int lvae_wgrad_unpack_batched(const void* desc_dev, int n, int max_n_real, lvae_stream_t stream);
-/* Same with per-channel reductions fused into the epilogue (bf16 output, N == 64, no residual / split):
- *   stats_acc  [2*64] += sum / sum-of-squares of the output as stored (the next BatchNorm's statistics),
+/* Same with per-channel reductions fused into the epilogue (bf16 output, N == 64, no split):
+ *   stats_acc  [2*64] += sum / sum-of-squares of the output as stored (the next BatchNorm's statistics); with res, of
+ *              bf16((acc + bias) * out_scale + res): the second conv of an ungated residual block (lib/nn.py:62-99, the
+ *              residual add of :99) hands its output's statistics to the next block's first BatchNorm (resident weights
+ *              only; N != 64, fp32 output, a split output or streamed weights are rejected before any device call),
  *   bnb_*      BatchNorm-backward sums over this data-gradient output dy: bnb_acc [2*64] += sum(g), sum(g*xhat) with
  *              xhat = (bnb_x - mean)*rstd, g = dy * act'(xhat*gamma + beta); bnb_save = [mean | rstd]. */
 typedef struct {

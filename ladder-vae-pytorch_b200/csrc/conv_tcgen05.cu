@@ -61,7 +61,7 @@ struct TcParams {
   const __nv_bfloat16* gate_x;
   int gate_act;
   int gate_skip_h;          // eval mode: h = [a | g] is only staged for the gate pass, never stored (nothing runs backward)
-  int tma_store;            // bf16 output, N % 64 == 0, no residual: epilogue stages the tile in smem and stores it with TMA
+  int tma_store;            // bf16 output, N % 64 == 0 (residual: resident weights): epilogue stages the tile in smem, TMA store
   // eval-mode BatchNorm + activation of the CONSUMER folded into this conv's epilogue (FUSE 4, N == 64, no_grad callers):
   // y = act((acc + bias) * s + (beta - mean * s)), s = gamma * rsqrt(var + eps) -- derived in the prologue from the running
   // statistics, so the separate BatchNorm-apply pass (one read + one write of the tensor, one launch) disappears
@@ -135,7 +135,9 @@ __device__ __forceinline__ void epilogue16(const uint32_t* __restrict__ r, const
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           float2 f0 = __bfloat1622float2(h0[j]), f1 = __bfloat1622float2(h1[j]);
-          v[2 * j] += f0.x; v[2 * j + 1] += f0.y; v[8 + 2 * j] += f1.x; v[8 + 2 * j + 1] += f1.y;
+          // no FMA contraction with the scale: the same arithmetic as the TMA-store epilogue
+          v[2 * j] = __fadd_rn(v[2 * j], f0.x); v[2 * j + 1] = __fadd_rn(v[2 * j + 1], f0.y);
+          v[8 + 2 * j] = __fadd_rn(v[8 + 2 * j], f1.x); v[8 + 2 * j + 1] = __fadd_rn(v[8 + 2 * j + 1], f1.y);
         }
       }
       uint4 w0, w1;
@@ -151,7 +153,7 @@ __device__ __forceinline__ void epilogue16(const uint32_t* __restrict__ r, const
     } else {
 #pragma unroll
       for (int j = 0; j < 16; ++j)
-        if (j < nvalid) o[j] = __float2bfloat16(v[j] + (rr ? __bfloat162float(rr[j]) : 0.f));
+        if (j < nvalid) o[j] = __float2bfloat16(__fadd_rn(v[j], rr ? __bfloat162float(rr[j]) : 0.f));
     }
   }
 }
@@ -166,7 +168,9 @@ __device__ __forceinline__ void epilogue16(const uint32_t* __restrict__ r, const
 // ACT (FUSE 2 / 3 only): the activation of the fused BatchNorm-backward / gate pass as a compile-time constant (ACT_ELU, the
 // model default) or -1 = runtime value; a switch inside the unrolled second pass costs one jump table per element.
 // SW: streamed weights (FUSE == 0, non-halo tiles only): no resident weight block, stage = A box + B tile.
-template <int FUSE, int ACT = -1, bool SW = false>
+// RES: residual added on the TMA-store path (FUSE 0 / 1, resident weights); a variant of its own, so that the kernels without a
+// residual carry neither its registers nor its loads.
+template <int FUSE, int ACT = -1, bool SW = false, bool RES = false>
 __global__ void __launch_bounds__(FUSE == 4 ? TC_THREADS + 160 : TC_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
                const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmY,
@@ -452,6 +456,19 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
       const bool valid = m < p.M_total;
       const long long rbase = row_base(tile);
       if (FUSE == 2) load_xq(rbase);                               // BatchNorm input rows: fetched while the MMAs still run
+      // residual of the TMA-store path (bf16, N <= 128): this thread's row, its (at most two) 32-column chunks, requested
+      // while the MMAs still run
+      constexpr int NCH = (FUSE == 1 || FUSE == 2 || FUSE == 4) ? 1 : 2;
+      uint4 rq[RES ? NCH : 1][4];
+      if constexpr (RES) {
+#pragma unroll
+        for (int nch = 0; nch < NCH; ++nch) {
+          const int c0 = 32 * half + 64 * nch;
+          const uint4* src = reinterpret_cast<const uint4*>((const __nv_bfloat16*)p.res + m * p.N + c0);
+#pragma unroll
+          for (int q = 0; q < 4; ++q) rq[nch][q] = (valid && c0 < p.Npad) ? __ldg(src + q) : make_uint4(0u, 0u, 0u, 0u);
+        }
+      }
       mbar_wait(BAR(2 * S + 1 + buf), use & 1);
       tc_fence_after();
       if (p.dbg && blockIdx.x == 0 && warp == 2 && lane == 0) p.dbg[it * 8 + 4] = clock64();
@@ -459,8 +476,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
       const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * p.Npad);
       const float* scale_row = p.out_scale ? p.out_scale + (long long)b * p.N : nullptr;
       if (FUSE != 0 || p.tma_store) {
-        // ---- TMEM -> registers (bias, Dropout2d scale, bf16 pack), release the accumulator, stage in smem, TMA store ----
-        constexpr int NCH = (FUSE == 1 || FUSE == 2 || FUSE == 4) ? 1 : 2;       // fused reductions: N = 64, one chunk per thread
+        // ---- TMEM -> registers (bias, Dropout2d scale, residual, bf16 pack), release the accumulator, stage in smem, TMA
+        // store.  Fused reductions: N = 64, one chunk per thread ----
         uint4 packed[NCH][4];
 #pragma unroll
         for (int nch = 0; nch < NCH; ++nch) {                      // N <= 128 on this path: at most two chunks per thread
@@ -487,6 +504,19 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
             if (scale_row) {
               const float4 s4 = __ldg(reinterpret_cast<const float4*>(scale_row + c0 + 4 * q));
               f[4 * q] *= s4.x; f[4 * q + 1] *= s4.y; f[4 * q + 2] *= s4.z; f[4 * q + 3] *= s4.w;
+            }
+          }
+          if constexpr (RES) {
+            // bf16((acc + bias) * scale + res), rounded once; __fadd_rn is never contracted into an FMA with the scale, so the
+            // sum is the fp32 output of the same launch without a residual, plus res
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const uint32_t w[4] = {rq[nch][q].x, rq[nch][q].y, rq[nch][q].z, rq[nch][q].w};
+#pragma unroll
+              for (int e = 0; e < 4; ++e) {
+                f[8 * q + 2 * e] = __fadd_rn(f[8 * q + 2 * e], __uint_as_float(w[e] << 16));
+                f[8 * q + 2 * e + 1] = __fadd_rn(f[8 * q + 2 * e + 1], __uint_as_float(w[e] & 0xFFFF0000u));
+              }
             }
           }
 #pragma unroll
@@ -719,7 +749,7 @@ LVAE_API int lvae_conv2d_tc(const void* x, const void* x2, const void* wp, const
 }
 
 // fuse (host struct, may be NULL): per-channel reductions computed in the epilogue, see LvaeConvFuse in include/lvae_b200.h.
-// Only on the TMA-store path (bf16 output, N == 64, no residual); anything else is rejected.
+// Only on the TMA-store path (bf16 output, N == 64; a residual only with the output statistics); anything else is rejected.
 LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, const float* bias, const float* out_scale,
                                const void* res, void* y, void* y2, int nsplit, int B, int H, int W, int Cin, int N,
                                int ksize, int flip, int out_f32, const LvaeConvFuse* fuse, cudaStream_t stream) {
@@ -768,6 +798,9 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   const int wplan = tc_weight_plan(Cin, N, ksize, inputs, H, W, out_f32);
   LVAE_REQUIRE(wplan != 0, "conv2d_tc: weights leave no room for the activation pipeline");
   const bool stream_w = wplan == 2;
+  LVAE_REQUIRE(!(res && p.bnb_acc), "conv2d_tc: a residual cannot be combined with the fused BatchNorm-backward sums");
+  LVAE_REQUIRE(!(res && p.stats_acc) || (N == 64 && !out_f32 && !y2 && !stream_w),
+               "conv2d_tc: residual + fused output statistics need N == 64, bf16 output, no split output and resident weights");
   LVAE_REQUIRE(!stream_w || !fuse, "conv2d_tc: fused epilogues need resident weights");
   int kb = 0;
   for (int t = 0; t < taps; ++t) {
@@ -787,12 +820,13 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
   LVAE_REQUIRE(p.tmem_cols <= 512, "conv2d_tc: accumulator does not fit TMEM");
   const int max_smem = TC_MAX_SMEM;
   const int wbytes = stream_w ? 0 : ((p.n_kb * p.Npad * 128) + 1023) & ~1023;
-  p.tma_store = (!out_f32 && N % 64 == 0 && N <= 128 && !res && (!y2 || nsplit % 64 == 0)) ? 1 : 0;
+  // a residual rides on the TMA-store path with resident weights (its loads are issued ahead of the accumulator wait)
+  p.tma_store = (!out_f32 && N % 64 == 0 && N <= 128 && (!res || !stream_w) && (!y2 || nsplit % 64 == 0)) ? 1 : 0;
   const int out_stage = p.tma_store ? (p.Npad / 64 + (p.gate_x ? 1 : 0)) * TC_STAGE_BYTES : 0;
   LVAE_REQUIRE(!p.gate_x || p.tma_store, "conv2d_tc: the gated-residual epilogue needs the TMA-store path");
   LVAE_REQUIRE(!p.fold_gamma || p.tma_store, "conv2d_tc: the folded BatchNorm epilogue needs the TMA-store path");
   LVAE_REQUIRE(!(p.stats_acc || p.bnb_acc) || (p.tma_store && (N == 64 || p.gate_x) && !y2),
-               "conv2d_tc: fused reductions need the TMA-store path (bf16 output, N == 64, no residual, no split)");
+               "conv2d_tc: fused reductions need the TMA-store path (bf16 output, N == 64, no split)");
   p.halo = (!stream_w && ksize == 3 && !x2 && Cin == 64 && W % 8 == 0 && H % 16 == 0 &&
             (max_smem - wbytes - out_stage) / (18 * 16 * 128) >= 2) ? 1 : 0;
   p.stage_bytes = 18 * 16 * 128;
@@ -849,19 +883,24 @@ LVAE_API int lvae_conv2d_tc_ex(const void* x, const void* x2, const void* wp, co
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<4, ACT_ELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<0, -1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<0, -1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<1, -1, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e != cudaSuccess) { lvae_set_error("conv2d_tc: cannot raise dynamic smem: %s", cudaGetErrorString(e)); return LVAE_ERR_CUDA; }
     attr_smem = 227 * 1024;
   }
   const int n_tiles = p.halo ? B * p.tiles_per_img : (p.M_total + TC_BM - 1) / TC_BM;
   const int grid = n_tiles < lvae_num_sms() ? n_tiles : lvae_num_sms();
+  const bool res_tma = res && p.tma_store;     // (the gated-residual, folded and BatchNorm-backward epilogues reject res)
   if (p.fold_gamma && p.fold_act == ACT_ELU) lvae_launch(conv_tc_kernel<4, ACT_ELU>, grid, TC_THREADS + 160, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.fold_gamma) lvae_launch(conv_tc_kernel<4>, grid, TC_THREADS + 160, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.gate_x && p.gate_act == ACT_ELU) lvae_launch(conv_tc_kernel<3, ACT_ELU>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.gate_x) lvae_launch(conv_tc_kernel<3>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
+  else if (p.stats_acc && res_tma) lvae_launch(conv_tc_kernel<1, -1, false, true>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.stats_acc) lvae_launch(conv_tc_kernel<1>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.bnb_acc && p.bnb_act == ACT_ELU) lvae_launch(conv_tc_kernel<2, ACT_ELU>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (p.bnb_acc) lvae_launch(conv_tc_kernel<2>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else if (stream_w) lvae_launch(conv_tc_kernel<0, -1, true>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
+  else if (res_tma) lvae_launch(conv_tc_kernel<0, -1, false, true>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   else lvae_launch(conv_tc_kernel<0>, grid, TC_THREADS, smem, stream, tmA0, tmA1, tmW, tmY, tmY2, p);
   LVAE_COUNT_LAUNCH();
   LVAE_CHECK_LAUNCH("conv2d_tc");

@@ -994,7 +994,7 @@ __global__ void bn_act_fwd2_kernel(const TI* __restrict__ x, TO* __restrict__ y,
 
 // GATE: the gate backward of the residual block that PRODUCED x (the next block of the backward pass) rides in the same pass --
 // dx of this BatchNorm (+ residual gradient) is exactly that block's output gradient: dh = gate'(dx, gh) is written next to dx,
-// one launch and one re-read of dx less per pair of adjacent blocks (ops.GatedBlockFn hands the pending apply over).
+// one launch and one re-read of dx less per pair of adjacent blocks (ops.ResidualBlockFn hands the pending apply over).
 template <typename T, int V, int ACT = -1, bool GATE = false>
 __global__ void __launch_bounds__(256, GATE ? 2 : 3) bn_act_bwd2_kernel(const T* __restrict__ dy, const T* __restrict__ x, T* __restrict__ dx,
                                    const float* __restrict__ save, const float* __restrict__ gamma,

@@ -198,11 +198,16 @@ class ResidualBlock(nn.Module):
             layers.append(GateLayer2d(channels, 1, nonlin))
         self.block = nn.Sequential(*layers)
         self._plan = self._make_plan(list(self.block))
-        # the default block (BN, act, conv, dropout) x 2 + gate runs as ONE autograd node with a hand-made backward
-        kinds = [(k, m is not None, a is not None) for k, m, a in self._plan]
-        self._whole_block = kinds == [("bnact", True, True), ("conv", True, True), ("bnact", True, True),
-                                      ("conv", True, True), ("gate", True, False)] and \
-            self._plan[0][2] == self._plan[2][2]
+        self._whole_block = self.takes_block_node(self._plan)
+
+    @staticmethod
+    def takes_block_node(plan) -> bool:
+        """(BN, act, conv, [dropout]) x 2 [+ gate] -- 'bacdbacd' and 'bacdbac', gated or not, with a Dropout2d behind either
+        conv, both or neither, and the same activation in both BatchNorm + activation steps -- runs as ONE autograd node
+        with a hand-made backward (ops.residual_block).  'cabdcabd' and batchnorm=False run step by step."""
+        kinds = [k for k, _, _ in plan]
+        return (kinds in (["bnact", "conv", "bnact", "conv"], ["bnact", "conv", "bnact", "conv", "gate"])
+                and plan[0][1] is not None and plan[2][1] is not None and plan[0][2] == plan[2][2])
 
     @staticmethod
     def _make_plan(mods):
@@ -243,7 +248,8 @@ class ResidualBlock(nn.Module):
             return self.block(x) + x
         if self._whole_block and ops.whole_block_enabled():
             p = self._plan
-            return ops.gated_block(x, p[0][1], p[1][1], p[1][2], p[2][1], p[3][1], p[3][2], p[4][1], p[0][2])
+            return ops.residual_block(x, p[0][1], p[1][1], p[1][2], p[2][1], p[3][1], p[3][2], p[4][1] if len(p) == 5 else None,
+                                      p[0][2])
         h, last = x, len(self._plan) - 1
         for idx, (kind, m, aux) in enumerate(self._plan):
             if kind == "bnact":

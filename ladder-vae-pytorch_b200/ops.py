@@ -550,9 +550,10 @@ def wgrad_tc_windows(N: int, k: int, two_inputs: bool, xC: int):
     return tuple((x0, n, c0) for x0 in range(0, xC, 64) for n, c0 in wgrad_tc_plan(N, k, two_inputs))
 
 
-def _tc_fusable(N, out_f32, res, nsplit=0) -> bool:
-    """Can the conv's epilogue carry a fused per-channel reduction (TMA-store path of lvae_conv2d_tc)?"""
-    return N == 64 and not out_f32 and res is None and not nsplit
+def _tc_fusable(N, out_f32, nsplit=0) -> bool:
+    """Can the conv's epilogue carry a fused per-channel reduction (TMA-store path of lvae_conv2d_tc, with or without a
+    residual)?"""
+    return N == 64 and not out_f32 and not nsplit
 
 
 def _conv_tc(x, x2, wp, bias, out_scale, res, N, ksize, flip, out_f32, nsplit=0, stats_acc=None, bnb=None, gate=None, fold=None):
@@ -566,8 +567,13 @@ def _conv_tc(x, x2, wp, bias, out_scale, res, N, ksize, flip, out_f32, nsplit=0,
         y2 = torch.empty((B, H, W, N - nsplit), dtype=odt, device=x.device)
     else:
         y, y2 = torch.empty((B, H, W, N), dtype=odt, device=x.device), None
-    if conv_tc_plan(C, N, ksize, x2 is not None, H, W, out_f32) == TC_STREAMED:
+    streamed = conv_tc_plan(C, N, ksize, x2 is not None, H, W, out_f32) == TC_STREAMED
+    if streamed:
         key = "tc_dgrad_streamed" if flip else "tc_fwd_streamed"
+        stats[key] = stats.get(key, 0) + 1
+    if res is not None and not out_f32:
+        # bf16 residual: added in the TMA-store epilogue (resident weights, N % 64 == 0, N <= 128), else by scattered row stores
+        key = "res_tma" if (N % 64 == 0 and N <= 128 and not streamed) else "res_scattered"
         stats[key] = stats.get(key, 0) + 1
     fuse = None
     gate_out = None
@@ -639,7 +645,7 @@ def conv_forward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, resn, sta
     if spec.tc_forward_ok(xn, x2n) and (resn is None or resn.dtype == (torch.float32 if want_f32 else torch.bfloat16)):
         wp = spec.pack_tc_fwd.get(weight, torch.bfloat16)
         stats["tc_fwd"] += 1
-        fused = stats_acc is not None and _tc_fusable(spec.cout, want_f32, resn)
+        fused = stats_acc is not None and _tc_fusable(spec.cout, want_f32)
         y = _conv_tc(xn, x2n, wp, bias, out_scale, resn, spec.cout, spec.k, False, want_f32,
                      stats_acc=stats_acc if fused else None)
         return (y, fused) if stats_acc is not None else y
@@ -694,7 +700,7 @@ def conv_backward_raw(spec: ConvSpec, xn, x2n, weight, bias, out_scale, gyn, nee
             wpb = spec.pack_tc_bwd.get(weight, torch.bfloat16)
             stats["tc_dgrad"] += 1
             if x2n is None:
-                fuse_bnb = bnb is not None and not padded and _tc_fusable(spec.cin, False, None)
+                fuse_bnb = bnb is not None and not padded and _tc_fusable(spec.cin, False)
                 # padded (conv_out of a stochastic block reading the 64-channel bf16 copy of z): the gradient goes to the
                 # fp32, Z-channel z the autograd graph holds -> fp32 epilogue, no padding channels
                 gx = _conv_tc(gyn, None, wpb, None, dx_scale, None, spec.cin, spec.k, True, padded,
@@ -903,7 +909,7 @@ def bn_act(x, bn, act_id: int, out_dtype=None):
 BN_STRIPES = 8
 _bn_epoch = [0]
 _whole_block = [True]
-_gate_keep_h = [True]     # set per call by gated_block(): autograd.Function.forward always runs with grad mode off
+_gate_keep_h = [True]     # set per call by residual_block(): autograd.Function.forward always runs with grad mode off
 # Fused paths of the gated blocks.  Always on: they are flags only so that tests/test_conv_gate_gpu.py and
 # tests/test_block_stack_fusion_gpu.py can turn them off for their reference runs.
 # _gate_chain: conv2 + gate conv + gate as ONE launch, the 1x1 GEMM reading the staged conv2 tile (lvae_conv_gate_tc; on a
@@ -989,13 +995,16 @@ def _bn_clean(bn, acc_rows, which: str):
     setattr(bn, attr, _bn_epoch[0])
 
 
-class GatedBlockFn(Function):
-    """One whole ResidualGatedBlock of type 'bacdbacd' (lib/nn.py:78-99 + GateLayer2d :108-126) with a hand-made
-    backward schedule:
+class ResidualBlockFn(Function):
+    """One whole ResidualBlock of type 'bacdbacd' or 'bacdbac' (lib/nn.py:62-99), gated (+ GateLayer2d :108-126) or not,
+    with a hand-made backward schedule.  mask1 / mask2 are the Dropout2d masks behind conv1 / conv2 (either may be None).
+    Gated:
         forward : [stats] BN1+act -> conv1 (*mask1) -> stats, BN2+act -> conv2 (*mask2) -> 1x1 gate conv ->
                   act(a)*sigmoid(b) + x  (+ statistics of the output for the next block's BN1)
         backward: gate' -> 1x1 dgrad (*mask2 in its epilogue) / wgrad -> conv2 dgrad / wgrad -> BN2' (*mask1 fused)
                   -> conv1 dgrad / wgrad -> BN1' (+ residual gradient fused)
+    Ungated (gate conv None): conv2 (*mask2) + x in one epilogue, which also accumulates the output statistics; backward
+        gout * mask2 -> conv2 dgrad / wgrad -> BN2' (*mask1 fused) -> conv1 dgrad / wgrad -> BN1' (+ residual gradient fused)
     Dropout2d masks are folded into neighbouring kernels' epilogues and BatchNorm needs no finalize / parameter kernels."""
 
     @staticmethod
@@ -1052,36 +1061,51 @@ class GatedBlockFn(Function):
             y1 = conv_forward_raw(conv1.spec, a1, None, w1, cb1, m1, None)
         if not fold2:
             a2 = bn_fwd(y1, bn2, sc2, saves[1], g2, b2, acc2)
-        gspec = gconv.spec
-        # conv2, the 1x1 gate conv and the gate itself as one launch (csrc/conv_gate_tcgen05.cu)
-        chain = (_gate_chain[0] and C == 64 and gspec.cout == 128 and gspec.k == 1 and conv2.spec.k == 3 and conv2.spec.cout == 64
-                 and xn.dtype == torch.bfloat16 and not gspec.out_fp32 and not conv2.spec.out_fp32
-                 and conv2.spec.tc_forward_ok(a2, None) and gspec.tc_forward_ok(a2, None)
-                 and (m2 is None or (m2.dtype == torch.float32 and m2.is_contiguous())))
-        y2 = None if chain else conv_forward_raw(conv2.spec, a2, None, w2, cb2, m2, None)
-        out_stats = None
-        if training and 256 % (C // 4) == 0:
-            out_stats = sc1[2]                        # statistics of this block's output, for the next block's BN1
-            _bn_clean(bn1, out_stats, "out")
-        if chain:
-            stats["tc_fwd"] += 2
-            stats["gate_chain"] = stats.get("gate_chain", 0) + 1
-            y2, h, out = _conv_gate_chain(a2, conv2.spec.pack_tc_fwd.get(w2, torch.bfloat16), cb2, m2,
-                                          gspec.pack_tc_fwd.get(wg, torch.bfloat16), gbias, xn, gact, out_stats, _gate_keep_h[0])
-        elif (C == 64 and gspec.cout == 128 and xn.dtype == torch.bfloat16 and not gspec.out_fp32
-                and gspec.tc_forward_ok(y2, None)):
-            # gate, residual add and the output statistics ride in the epilogue of the 1x1 gate conv
-            stats["tc_fwd"] += 1
-            stats["gate_fused"] = stats.get("gate_fused", 0) + 1
-            h, out = _conv_tc(y2, None, gspec.pack_tc_fwd.get(wg, torch.bfloat16), gbias, None, None, 128, gspec.k, False, False,
-                              stats_acc=out_stats, gate=(xn, gact))
-        else:
-            h = conv_forward_raw(gspec, y2, None, wg, gbias, None, None)
-            out = torch.empty_like(xn)
-            if out_stats is not None:
-                call("lvae_gate_fwd_stats", h.data_ptr(), xn.data_ptr(), out.data_ptr(), out_stats.data_ptr(), Pn, C, gact, dt, _stream())
+        out_stats = y2 = h = None
+        if gconv is None:
+            # ungated: out = conv2(a2) * mask2 + x, the residual added in the TMA-store epilogue; in training the same epilogue
+            # accumulates the statistics of out for the next block's BN1 (bf16, 64 channels: free there -- elsewhere the
+            # consumer's BatchNorm computes them)
+            if (training and C == 64 and xn.dtype == torch.bfloat16 and not conv2.spec.out_fp32
+                    and conv2.spec.tc_forward_ok(a2, None)):
+                out_stats = sc1[2]
+                _bn_clean(bn1, out_stats, "out")
+                out, fused = conv_forward_raw(conv2.spec, a2, None, w2, cb2, m2, xn, stats_acc=out_stats)
+                if not fused:
+                    call("lvae_bn_stats", out.data_ptr(), out_stats.data_ptr(), Pn, C, dt, _stream())
             else:
-                call("lvae_gate_fwd", h.data_ptr(), xn.data_ptr(), out.data_ptr(), Pn, C, gact, dt, _stream())
+                out = conv_forward_raw(conv2.spec, a2, None, w2, cb2, m2, xn)
+        else:
+            gspec = gconv.spec
+            # conv2, the 1x1 gate conv and the gate itself as one launch (csrc/conv_gate_tcgen05.cu)
+            chain = (_gate_chain[0] and C == 64 and gspec.cout == 128 and gspec.k == 1 and conv2.spec.k == 3 and conv2.spec.cout == 64
+                     and xn.dtype == torch.bfloat16 and not gspec.out_fp32 and not conv2.spec.out_fp32
+                     and conv2.spec.tc_forward_ok(a2, None) and gspec.tc_forward_ok(a2, None)
+                     and (m2 is None or (m2.dtype == torch.float32 and m2.is_contiguous())))
+            if not chain:
+                y2 = conv_forward_raw(conv2.spec, a2, None, w2, cb2, m2, None)
+            if training and 256 % (C // 4) == 0:
+                out_stats = sc1[2]                        # statistics of this block's output, for the next block's BN1
+                _bn_clean(bn1, out_stats, "out")
+            if chain:
+                stats["tc_fwd"] += 2
+                stats["gate_chain"] = stats.get("gate_chain", 0) + 1
+                y2, h, out = _conv_gate_chain(a2, conv2.spec.pack_tc_fwd.get(w2, torch.bfloat16), cb2, m2,
+                                              gspec.pack_tc_fwd.get(wg, torch.bfloat16), gbias, xn, gact, out_stats, _gate_keep_h[0])
+            elif (C == 64 and gspec.cout == 128 and xn.dtype == torch.bfloat16 and not gspec.out_fp32
+                    and gspec.tc_forward_ok(y2, None)):
+                # gate, residual add and the output statistics ride in the epilogue of the 1x1 gate conv
+                stats["tc_fwd"] += 1
+                stats["gate_fused"] = stats.get("gate_fused", 0) + 1
+                h, out = _conv_tc(y2, None, gspec.pack_tc_fwd.get(wg, torch.bfloat16), gbias, None, None, 128, gspec.k, False, False,
+                                  stats_acc=out_stats, gate=(xn, gact))
+            else:
+                h = conv_forward_raw(gspec, y2, None, wg, gbias, None, None)
+                out = torch.empty_like(xn)
+                if out_stats is not None:
+                    call("lvae_gate_fwd_stats", h.data_ptr(), xn.data_ptr(), out.data_ptr(), out_stats.data_ptr(), Pn, C, gact, dt, _stream())
+                else:
+                    call("lvae_gate_fwd", h.data_ptr(), xn.data_ptr(), out.data_ptr(), Pn, C, gact, dt, _stream())
         ctx.save_for_backward(xn, a1, y1, a2, y2, h, saves, g1, b1, w1, cb1, g2, b2, w2, cb2, wg, gbias, m1, m2)
         ctx.blk, ctx.training = blk, training
         ctx.defer_bn1 = bool(_defer_bn1_next[0])
@@ -1100,32 +1124,38 @@ class GatedBlockFn(Function):
         if gn.dtype != xn.dtype:
             gn = gn.to(xn.dtype)
         ng = ctx.needs_input_grad
-        gsp = gconv.spec
-        # gate
-        dh = torch.empty_like(h)
-        pend = _pending_bn1.pop(gn.data_ptr(), None)
-        if pend is not None:
-            # the consumer block deferred its BatchNorm1-backward apply: gn is its (still uncomputed) dx -- one pass writes
-            # dx into gn and this block's gate gradient dh
-            assert pend["shape"] == tuple(gn.shape) and gn.dtype == torch.bfloat16 and h.dtype == torch.bfloat16
-            grad_site()
-            pdg, _ = _param_grad_buffer(pend["gamma"])
-            pdb, _ = _param_grad_buffer(pend["beta"])
-            stats["bn1_gate_fused"] = stats.get("bn1_gate_fused", 0) + 1
-            call("lvae_bn_act_bwd2_gate", pend["dy"].data_ptr(), pend["x"].data_ptr(), gn.data_ptr(), pend["save"].data_ptr(),
-                 pend["gamma"].data_ptr(), pend["beta"].data_ptr(), pend["acc"].data_ptr(), pdg.data_ptr(), pdb.data_ptr(), None,
-                 pend["add"].data_ptr(), h.data_ptr(), dh.data_ptr(), Pn, H * W, C, pend["act"], gact,
-                 1 if pend["training"] else 0, _stream())
+        if gconv is None:
+            # ungated: the gradient wrt conv2's raw output is gout * mask2 (applied by conv_backward_raw); never handed a
+            # deferred BatchNorm1 apply (residual_block marks only gated blocks' outputs private)
+            dy2, scale2, gwg, ggb = gn, m2, None, None
         else:
-            call("lvae_gate_bwd", gn.data_ptr(), h.data_ptr(), dh.data_ptr(), Pn, C, gact, dt, _stream())
-        # 1x1 gate conv: dgrad carries conv2's Dropout2d mask in its epilogue -> gradient wrt conv2's raw output
-        dy2, _, gwg, ggb = conv_backward_raw(gsp, y2, None, wg, gbias, None, dh, True, ng[9], ng[10], dx_scale=m2)
+            gsp = gconv.spec
+            # gate
+            dh = torch.empty_like(h)
+            pend = _pending_bn1.pop(gn.data_ptr(), None)
+            if pend is not None:
+                # the consumer block deferred its BatchNorm1-backward apply: gn is its (still uncomputed) dx -- one pass writes
+                # dx into gn and this block's gate gradient dh
+                assert pend["shape"] == tuple(gn.shape) and gn.dtype == torch.bfloat16 and h.dtype == torch.bfloat16
+                grad_site()
+                pdg, _ = _param_grad_buffer(pend["gamma"])
+                pdb, _ = _param_grad_buffer(pend["beta"])
+                stats["bn1_gate_fused"] = stats.get("bn1_gate_fused", 0) + 1
+                call("lvae_bn_act_bwd2_gate", pend["dy"].data_ptr(), pend["x"].data_ptr(), gn.data_ptr(), pend["save"].data_ptr(),
+                     pend["gamma"].data_ptr(), pend["beta"].data_ptr(), pend["acc"].data_ptr(), pdg.data_ptr(), pdb.data_ptr(), None,
+                     pend["add"].data_ptr(), h.data_ptr(), dh.data_ptr(), Pn, H * W, C, pend["act"], gact,
+                     1 if pend["training"] else 0, _stream())
+            else:
+                call("lvae_gate_bwd", gn.data_ptr(), h.data_ptr(), dh.data_ptr(), Pn, C, gact, dt, _stream())
+            # 1x1 gate conv: dgrad carries conv2's Dropout2d mask in its epilogue -> gradient wrt conv2's raw output
+            dy2, _, gwg, ggb = conv_backward_raw(gsp, y2, None, wg, gbias, None, dh, True, ng[9], ng[10], dx_scale=m2)
+            scale2 = None
         sc1b, sc2b = bn_scratch(bn1, dev), bn_scratch(bn2, dev)
         acc1b, acc2b = sc1b[1], sc2b[1]
         _bn_clean(bn1, acc1b, "bwd")
         _bn_clean(bn2, acc2b, "bwd")
-        # conv2 (dy2 is already masked); its dgrad epilogue also accumulates BN2's backward sums
-        da2, _, gw2, gcb2 = conv_backward_raw(conv2.spec, a2, None, w2, cb2, None, dy2, True, ng[7], ng[8],
+        # conv2 (dy2 is masked, or scale2 masks it); its dgrad epilogue also accumulates BN2's backward sums
+        da2, _, gw2, gcb2 = conv_backward_raw(conv2.spec, a2, None, w2, cb2, scale2, dy2, True, ng[7], ng[8],
                                               bnb=(y1, saves[1], g2, b2, acc2b, act) if C == 64 else None)
         fused2 = conv_backward_raw.last_fused
 
@@ -1156,9 +1186,11 @@ class GatedBlockFn(Function):
         return (as_nchw(dx), gg1, gb1, gw1, gcb1, gg2, gb2, gw2, gcb2, gwg, ggb, None, None, None, None, None)
 
 
-def gated_block(x, bn1, conv1, drop1, bn2, conv2, drop2, gate_layer, act_id):
+def residual_block(x, bn1, conv1, drop1, bn2, conv2, drop2, gate_layer, act_id):
+    """A 'bacdbacd' / 'bacdbac' residual block as one autograd node (ResidualBlockFn).  drop1 / drop2: the Dropout2d modules
+    behind conv1 / conv2, or None; gate_layer: the GateLayer2d of a gated block, None for an ungated one."""
     training = bn1.training
-    # statistics of x computed by the kernel that produced it (previous block's gate), if still valid
+    # statistics of x computed by the kernel that produced it (previous block's last epilogue), if still valid
     x_stats = None
     st = getattr(x, "_lvae_stats", None)
     if training and st is not None and st[2] == _bn_epoch[0] and st[1] == x.shape[0] * x.shape[2] * x.shape[3]:
@@ -1169,17 +1201,22 @@ def gated_block(x, bn1, conv1, drop1, bn2, conv2, drop2, gate_layer, act_id):
         m1 = m1.reshape(x.shape[0], -1)
     if m2 is not None:
         m2 = m2.reshape(x.shape[0], -1)
-    blk = (bn1, bn2, conv1, conv2, gate_layer.conv, act_id, getattr(gate_layer.nonlin, "act_id", 0))
+    gconv = gate_layer.conv if gate_layer is not None else None
+    blk = (bn1, bn2, conv1, conv2, gconv, act_id, getattr(gate_layer.nonlin, "act_id", 0) if gate_layer is not None else 0)
     _gate_keep_h[0] = torch.is_grad_enabled()
-    private = _private_out[0]             # this block's output goes to the next gated block of the stack and nowhere else
+    # this block's output goes to the next block of the stack and nowhere else; only a gated block's backward picks the next
+    # block's deferred BatchNorm1 apply up (lvae_bn_act_bwd2_gate), so only its output is marked private
+    private = _private_out[0] and gconv is not None
     _private_out[0] = False
     # x is such a private output of the previous block: this block's BatchNorm1-backward apply may be handed over to it
     _defer_bn1_next[0] = bool(getattr(x, "_lvae_private", False)) and training and torch.is_grad_enabled() and x.requires_grad
     try:
-        out = GatedBlockFn.apply(x, bn1.weight, bn1.bias, conv1.weight, conv1.bias, bn2.weight, bn2.bias, conv2.weight,
-                                 conv2.bias, gate_layer.conv.weight, gate_layer.conv.bias, m1, m2, blk, x_stats, training)
+        out = ResidualBlockFn.apply(x, bn1.weight, bn1.bias, conv1.weight, conv1.bias, bn2.weight, bn2.bias, conv2.weight,
+                                    conv2.bias, gconv.weight if gconv is not None else None,
+                                    gconv.bias if gconv is not None else None, m1, m2, blk, x_stats, training)
     finally:
         _defer_bn1_next[0] = False            # never leaks into another block if the forward raised before reading it
+    stats["block_node"] = stats.get("block_node", 0) + 1
     if training and bn1._lvae_last_out_stats is not None:
         out._lvae_stats = bn1._lvae_last_out_stats
     if private and training and out.dtype == torch.bfloat16:
